@@ -4,6 +4,7 @@ fixture best_unet_model.pth, batch 64 x 3 x 512 x 512, bf16 tensor-core forward 
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's own CPU forward (oracle/_ref)
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's logits / masks as DIR/*.npy
 
 One process per GPU (torchrun for N > 1); images are independent, so ranks shard the batch
 with no data-path collective ("scaling": "weak": 64 images per GPU per step).  Rank 0 prints
@@ -35,6 +36,7 @@ if ROOT not in sys.path:
 METRIC = "unet_forward_images_per_sec"
 UNIT = "images/s"
 GFLOP_PER_IMAGE_512 = 385.406          # SURVEY.md 8(d): algorithmic FLOPs of the 23 convs at 512x512
+DUMP_BYTES = 64 * 10**6                # cap on everything --dump-outputs writes
 
 
 def layer_flops(layer, h, w) -> float:
@@ -145,6 +147,27 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "power_w_max": max(power) if power else None, "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(out_dir: str, outputs: dict, seed: int = 0):
+    """`--dump-outputs`: write the outputs of one step (name -> tensor [N, ...]) as out_dir/<name>.npy in float32, so
+    that two builds can be compared output for output.  Whole images are written: all N when they fit DUMP_BYTES,
+    otherwise a fixed seeded sample of batch positions, the same for every output (sorted, in
+    out_dir/image_index.npy).  Returns those positions."""
+    import numpy as np
+    import torch
+    n = len(next(iter(outputs.values())))
+    per_image = sum(t[0].numel() for t in outputs.values()) * 4
+    k = min(n, (DUMP_BYTES - 8 * n - 128 * (len(outputs) + 1)) // per_image)     # .npy headers: 128 bytes each
+    if k < 1:
+        raise ValueError(f"--dump-outputs: the outputs of one image ({per_image} bytes) exceed {DUMP_BYTES} bytes")
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "image_index.npy"), idx.astype(np.float64))
+    for name, t in outputs.items():
+        rows = t.index_select(0, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(out_dir, name + ".npy"), rows.float().cpu().numpy())
+    return idx
 
 
 def cpu_forward(state):
@@ -266,7 +289,15 @@ def main():
                     help="idle seconds before the end-to-end region's warm-up (same power state as the device-timed region's start)")
     ap.add_argument("--e2e-chunk", type=int, default=64,
                     help="images per forward inside the end-to-end call (copies of chunk i+1 overlap chunk i)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the logits and masks of the last timed step (rank 0) as DIR/logits.npy, DIR/mask.npy "
+                         "(float32, whole images: a fixed seeded sample of them, listed in DIR/image_index.npy, "
+                         "when all exceed 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -358,11 +389,16 @@ def main():
         step = g.replay
         for _ in range(args.warmup):
             step()
+    if args.dump_outputs:
+        logits.fill_(float("nan"))          # what is dumped must have been written by the timed steps
+        mask.fill_(255)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
     total_ms = timed(step, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"logits": logits, "mask": mask})
     launches_per_step = eng.last_launch_count()
     ms_per_step = total_ms / args.steps
     value = world * B / (ms_per_step / 1e3)
