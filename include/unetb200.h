@@ -36,11 +36,24 @@ enum {
 /* layer kinds in the packed-weights table */
 enum { UNETB200_STEM = 0, UNETB200_CONV3X3 = 1, UNETB200_CONVT2X2 = 2, UNETB200_HEAD = 3 };
 
-/* input formats accepted by unetb200_forward */
+/* input formats accepted by unetb200_forward.  The float formats are read as they are (no /255); a 16-bit element
+ * is widened to fp32 where the first conv reads it, which is exact, so fp16 / bf16 / NHWC input gives the same
+ * bits as the fp32 NCHW input x.float().contiguous().  NHWC = [N,H,W,C] in memory: the storage of a PyTorch
+ * channels_last [N,C,H,W] tensor.  Every input is 16-byte aligned (the tensor-core first conv reads it by TMA). */
 enum {
-    UNETB200_X_F32_NCHW = 0, /* float32 [N,C,H,W] in [0,1] -- what inference.preprocess returns (inference.py:36-42) */
-    UNETB200_X_U8_NHWC = 1   /* uint8 [N,H,W,C], scaled by /255 in the first kernel (inference.py:36) */
+    UNETB200_X_F32_NCHW = 0,  /* float32 [N,C,H,W] in [0,1] -- what inference.preprocess returns (inference.py:36-42) */
+    UNETB200_X_U8_NHWC = 1,   /* uint8 [N,H,W,C], scaled by /255 in the first kernel (inference.py:36) */
+    UNETB200_X_F16_NCHW = 2,  /* float16  [N,C,H,W] */
+    UNETB200_X_BF16_NCHW = 3, /* bfloat16 [N,C,H,W] */
+    UNETB200_X_F32_NHWC = 4,  /* float32  [N,H,W,C] */
+    UNETB200_X_F16_NHWC = 5,  /* float16  [N,H,W,C] */
+    UNETB200_X_BF16_NHWC = 6  /* bfloat16 [N,H,W,C] */
 };
+
+/* element type of the logits written by unetb200_forward_typed (and unetb200_conv3x3_head, wstat bits 3-4): the
+ * fp32 logits as computed, or rounded to nearest-even, i.e. z.to(torch.float16 / torch.bfloat16) bit for bit.
+ * Masks are decided on the fp32 value whatever the logits type. */
+enum { UNETB200_LOGITS_F32 = 0, UNETB200_LOGITS_F16 = 1, UNETB200_LOGITS_BF16 = 2 };
 
 /* A-operand staging strategy of the tensor-core conv kernel (see csrc/conv_tc.cuh) */
 enum { UNETB200_A_TAP = 0, UNETB200_A_COL3 = 1, UNETB200_A_HALO = 2,
@@ -144,6 +157,16 @@ int unetb200_forward_bits(unetb200_handle_t h, const void* x, int x_fmt, int n, 
                           void* workspace, uint64_t workspace_bytes, float* logits, uint8_t* mask_bits,
                           const float* logit_thr, void* stream);
 
+/* The forward of unetb200_forward / unetb200_forward_bits with the logits element type chosen per call:
+ *   logits       nullable; [N, n_classes, H, W] raw logits of type `logits_type` (UNETB200_LOGITS_*); 16-bit logits
+ *                are the fp32 logits rounded to nearest-even at the store
+ *   mask         nullable; byte masks as unetb200_forward (mask_bits = 0) or bit-packed as unetb200_forward_bits
+ *                (mask_bits = 1), decided on the fp32 logits
+ * An unknown x_fmt or logits_type is UNETB200_EINVAL. */
+int unetb200_forward_typed(unetb200_handle_t h, const void* x, int x_fmt, int n, int height, int width,
+                           void* workspace, uint64_t workspace_bytes, void* logits, int logits_type,
+                           uint8_t* mask, int mask_bits, const float* logit_thr, void* stream);
+
 /* Per-layer device times (ms) of the last forward run with option "profile" = 1.
  * Synchronises the stream's events.  `ms` has room for `count` floats. */
 int unetb200_layer_times(unetb200_handle_t h, float* ms, int count);
@@ -161,10 +184,11 @@ int unetb200_conv3x3(const void* src0, int c0, const void* src1, int c1, const v
                      const float* bias, int n, int height, int width, int cout, int relu, void* out,
                      void* pool_out, int bn, int amode, int wstat, void* stream);
 /* 3x3 conv (cout = 64) + ReLU with the 1x1 head and threshold fused into the epilogue.  `wstat` as above;
- * bit 2 makes `mask` the bit-packed [N, n_classes, H, W/8] format of unetb200_forward_bits. */
+ * bit 2 makes `mask` the bit-packed [N, n_classes, H, W/8] format of unetb200_forward_bits; bits 3-4 are the
+ * element type of `logits` (UNETB200_LOGITS_*, 0 = float32). */
 int unetb200_conv3x3_head(const void* src0, int c0, const void* w_packed, const float* bias,
                           const float* head_w, const float* head_b, int n_classes, int n, int height,
-                          int width, float* logits, uint8_t* mask, const float* logit_thr, int amode,
+                          int width, void* logits, uint8_t* mask, const float* logit_thr, int amode,
                           int wstat, void* stream);
 /* ConvTranspose2d(k=2,s=2): src [N,H,W,cin] bf16 -> out [N,2H,2W,cout] bf16. w_packed [4*cout][cin].
  * bn in {64,128,256}; bn | 0x1000 selects the CTA-pair variant. */

@@ -16,7 +16,8 @@ LIB_PATH = os.environ.get("UNETB200_LIB") or os.path.join(_HERE, "libunetb200.so
 
 OK, EINVAL, ECUDA, EARCH, ENOMEM = 0, 1, 2, 3, 4
 STEM, CONV3X3, CONVT2X2, HEAD = 0, 1, 2, 3
-X_F32_NCHW, X_U8_NHWC = 0, 1
+X_F32_NCHW, X_U8_NHWC, X_F16_NCHW, X_BF16_NCHW, X_F32_NHWC, X_F16_NHWC, X_BF16_NHWC = range(7)
+LOGITS_F32, LOGITS_F16, LOGITS_BF16 = 0, 1, 2
 A_TAP, A_COL3, A_HALO = 0, 1, 2
 
 
@@ -70,6 +71,7 @@ SYMBOLS = {
     "unetb200_workspace_bytes": (_U64, [_VP, _I, _I, _I]),
     "unetb200_forward": (_I, [_VP, _VP, _I, _I, _I, _I, _VP, _U64, _VP, _VP, C.POINTER(_F), _VP]),
     "unetb200_forward_bits": (_I, [_VP, _VP, _I, _I, _I, _I, _VP, _U64, _VP, _VP, C.POINTER(_F), _VP]),
+    "unetb200_forward_typed": (_I, [_VP, _VP, _I, _I, _I, _I, _VP, _U64, _VP, _I, _VP, _I, C.POINTER(_F), _VP]),
     "unetb200_layer_times": (_I, [_VP, C.POINTER(_F), _I]),
     "unetb200_last_launch_count": (_I, [_VP]),
     "unetb200_conv3x3": (_I, [_VP, _I, _VP, _I, _VP, _VP, _I, _I, _I, _I, _I, _VP, _VP, _I, _I, _I, _VP]),

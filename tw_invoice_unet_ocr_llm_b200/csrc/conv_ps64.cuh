@@ -46,7 +46,7 @@ constexpr int kPsW2 = 6 * 4096;                                   // image 2: si
 constexpr int kPsWBytes = kPsW1 + kPsW2;
 constexpr int kPsStatic = 64;
 
-template <int EPI, int X = 0>
+template <int EPI, int X = 0, int LT = LOGITS_F32>   // LT: logits element type of EPI_HEAD (conv_tc.cuh)
 __global__ void __launch_bounds__(384, 1) conv_ps64_kernel(const __grid_constant__ ConvParams p) {
     static_assert(EPI == EPI_STORE || EPI == EPI_STORE_POOL || EPI == EPI_HEAD, "phase-stacked kernel epilogues");
     extern __shared__ uint8_t smem_raw[];
@@ -266,7 +266,7 @@ __global__ void __launch_bounds__(384, 1) conv_ps64_kernel(const __grid_constant
                     for (int c = 0; c < NC; ++c) {
                         if (c < p.ncls && inside) {
                             const size_t o = ((static_cast<size_t>(n) * p.ncls + c) * p.H + y) * p.W + x;
-                            if (p.logits) *reinterpret_cast<float2*>(p.logits + o) = make_float2(z[0][c], z[1][c]);
+                            if (p.logits) store_logit2<LT>(p.logits, o, z[0][c], z[1][c]);
                             if (p.mask && !p.mask_bits)
                                 *reinterpret_cast<uchar2*>(p.mask + o) =
                                     make_uchar2(z[0][c] > p.thr[c] ? 1 : 0, z[1][c] > p.thr[c] ? 1 : 0);

@@ -44,7 +44,7 @@ constexpr int kRowAStage = (kRowItemBytes + 1023) / 1024 * 1024;
 constexpr int kRowBBlock = 64 * 128;                   // one tap of one K slice: 64 couts x 64 cin bf16
 constexpr int kRowStatic = 64;                         // static shared memory of the kernel (none; margin)
 
-template <int EPI, int X = 0>
+template <int EPI, int X = 0, int LT = LOGITS_F32>   // LT: logits element type of EPI_HEAD (conv_tc.cuh)
 __global__ void __launch_bounds__(384, 1) conv_row_kernel(const __grid_constant__ ConvParams p) {
     static_assert(EPI == EPI_STORE || EPI == EPI_STORE_POOL || EPI == EPI_HEAD, "row kernel epilogues");
     constexpr int R = kRowR;
@@ -264,7 +264,7 @@ __global__ void __launch_bounds__(384, 1) conv_row_kernel(const __grid_constant_
                         for (int c = 0; c < NC; ++c) {
                             if (c < p.ncls) {
                                 const size_t o = ((static_cast<size_t>(n) * p.ncls + c) * p.H + y) * p.W + px;
-                                if (p.logits) p.logits[o] = z[c];
+                                if (p.logits) store_logit<LT>(p.logits, o, z[c]);
                                 if (p.mask && !p.mask_bits) p.mask[o] = z[c] > p.thr[c] ? 1 : 0;
                             }
                         }

@@ -64,6 +64,7 @@
 // warps hand the accumulator back with remote mbarrier arrives.
 #pragma once
 #include "ptx.cuh"
+#include "stem.cuh"
 
 namespace ub {
 
@@ -71,6 +72,30 @@ enum : int { EPI_STORE = 0, EPI_STORE_POOL = 1, EPI_HEAD = 2, EPI_UPSAMPLE = 3 }
 enum : int { A_TAP = 0, A_COL3 = 1, A_HALO = 2, A_STEM = 3, A_STEMP = 4, A_ROW = 5 /* conv_row.cuh */, A_PHASE = 6 /* conv_phase.cuh */, A_PS64 = 7 /* conv_ps64.cuh */ };
 
 constexpr int kMaxClasses = 8;
+
+// element type of the logits the head epilogues write (include/unetb200.h UNETB200_LOGITS_*): fp32 as computed, or
+// the fp32 value rounded to nearest-even -- z.to(torch.float16 / torch.bfloat16) bit for bit.  The masks are always
+// decided on the fp32 value.
+enum : int { LOGITS_F32 = 0, LOGITS_F16 = 1, LOGITS_BF16 = 2 };
+
+template <int LT>
+__device__ __forceinline__ void store_logit(void* logits, size_t o, float z) {
+    if constexpr (LT == LOGITS_F32) static_cast<float*>(logits)[o] = z;
+    else if constexpr (LT == LOGITS_F16) static_cast<__half*>(logits)[o] = __float2half_rn(z);
+    else static_cast<__nv_bfloat16*>(logits)[o] = __float2bfloat16_rn(z);
+}
+// two horizontally adjacent pixels (o even): one 8-byte (fp32) or 4-byte (16-bit) store
+template <int LT>
+__device__ __forceinline__ void store_logit2(void* logits, size_t o, float z0, float z1) {
+    if constexpr (LT == LOGITS_F32) {
+        *reinterpret_cast<float2*>(static_cast<float*>(logits) + o) = make_float2(z0, z1);
+    } else if constexpr (LT == LOGITS_F16) {
+        *reinterpret_cast<__half2*>(static_cast<__half*>(logits) + o) = __halves2half2(__float2half_rn(z0), __float2half_rn(z1));
+    } else {
+        *reinterpret_cast<__nv_bfloat162*>(static_cast<__nv_bfloat16*>(logits) + o) =
+            __halves2bfloat162(__float2bfloat16_rn(z0), __float2bfloat16_rn(z1));
+    }
+}
 
 // Division by a launch constant as multiply-high + shift (dividends < 2^31): the per-tile index
 // arithmetic of every role (tile -> image / row / column, unit -> column block, ring slots) used ~20 %
@@ -113,7 +138,7 @@ struct ConvParams {
     const float* bias;       // [Cout] fp32 (BatchNorm-folded)
     const float* head_w;     // [ncls][64] fp32      (EPI_HEAD)
     const float* head_b;     // [ncls]               (EPI_HEAD)
-    float* logits;           // [N][ncls][H][W] fp32 (EPI_HEAD, nullable)
+    void* logits;            // [N][ncls][H][W], element type per the kernel's LT (EPI_HEAD, nullable)
     uint8_t* mask;           // [N][ncls][H][W] u8, or [N][ncls][H][W/8] bits when mask_bits (EPI_HEAD, nullable)
     int mask_bits;           // 1 = one bit per pixel: bit (x & 7) of byte x >> 3 of each row, LSB first
     float thr[kMaxClasses];  // logit-space thresholds
@@ -163,6 +188,12 @@ struct ConvCfg {
 constexpr int kStemSlots = 8;         // A_STEM: input-patch ring (TMA), slots of kStemSlotBytes
 constexpr int kStemSlotBytes = 3584;  //   fp32: [Cin <= 3][18][16] floats = 3456 B; uint8: [18][48] bytes
 constexpr int kStemPatchBytes = kStemSlots * kStemSlotBytes + 1024 + 2 * 2 * 3 * 180 * 4;   // ring + /255 table + split patches
+// every input box of the stem (stem.cuh stem_box_bytes, Cin <= 3) fits one ring slot; fp32 NCHW is the largest
+constexpr bool stem_boxes_fit(int f = 0) {
+    return f == kNumXFormats ? true : (stem_box_bytes(f, 3) <= kStemSlotBytes && stem_box_bytes(f, 1) <= kStemSlotBytes &&
+                                       stem_boxes_fit(f + 1));
+}
+static_assert(stem_boxes_fit(), "a stem input box exceeds its ring slot");
 constexpr int kOutStage = 16384;      // 128 pixels x 64 channels bf16
 constexpr int kPoolStage = 4096;      // 32 pixels x 64 channels bf16
 constexpr int kMaxRing = 8;           // upper bound on na and (non-stationary) nb
@@ -171,7 +202,9 @@ constexpr int kStaticSmem = 4096 + 64;   // s_bias (+ margin)
 constexpr int kSmemLimit = 232448;    // 227 KB per CTA on sm_100
 
 // X: A_STEM -> n_channels of the network input; EPI_HEAD -> n_classes (0 = generic, up to 8).
-template <int BN, int TAPS, int AMODE, int EPI, int X = 0, bool PAIR = false>
+// XF: A_STEM -> input format (stem.cuh X_*; X_RUNTIME = fp32 NCHW or uint8 NHWC by p.stem_fmt).
+// LT: EPI_HEAD -> logits element type (LOGITS_*).
+template <int BN, int TAPS, int AMODE, int EPI, int X = 0, bool PAIR = false, int XF = X_RUNTIME, int LT = LOGITS_F32>
 __global__ void __launch_bounds__(AMODE == A_STEM ? 640 : (AMODE == A_STEMP ? 512 : 384), 1)
 conv_tc_kernel(const __grid_constant__ ConvParams p) {
     constexpr int CIN = X;
@@ -182,6 +215,9 @@ conv_tc_kernel(const __grid_constant__ ConvParams p) {
     static_assert(AMODE != A_STEM || (TAPS == 1 && BN == 64 && CIN >= 1 && 9 * CIN < 32),
                   "stem: im2col rows of < 32 taps (one K slot carries the bias), 64 output channels");
     static_assert(EPI != EPI_HEAD || BN == 64, "fused head needs all 64 channels in one tile");
+    static_assert(XF == X_RUNTIME || (AMODE == A_STEM && XF != X_U8_NHWC && XF != X_F32_NCHW),
+                  "compile-time input formats: the new float formats of the im2col stem");
+    static_assert(LT == LOGITS_F32 || EPI == EPI_HEAD, "logits type of a head epilogue");
     using Cfg = ConvCfg<BN, TAPS, AMODE, PAIR>;
     constexpr int TPA = Cfg::TPA;
     constexpr int ITEMS = TAPS / TPA;
@@ -375,7 +411,7 @@ conv_tc_kernel(const __grid_constant__ ConvParams p) {
         // per group: two buffers of split (hi | lo) patch words
         uint32_t* s_split = reinterpret_cast<uint32_t*>(smem_gen + p.off_patch + kStemSlots * kStemSlotBytes + 1024) +
                             grp * 2 * PE;
-        if (p.stem_fmt != 0) {
+        if (XF == X_RUNTIME && p.stem_fmt != 0) {
             // uint8 ingest: k / 255.0f (inference.py:36, IEEE division) for all 256 byte values, once per CTA
             s_lut[threadIdx.x - 384] = __fdiv_rn(static_cast<float>(threadIdx.x - 384), 255.0f);
             named_bar_sync(11, 256);
@@ -386,11 +422,11 @@ conv_tc_kernel(const __grid_constant__ ConvParams p) {
              t += 2 * static_cast<int>(gridDim.x), it += 2) {
             const uint32_t slot = it % kStemSlots, ph = (it / kStemSlots) & 1;
             int sh = 3;                                          // first used column of the patch rows (floats)
-            if (p.stem_fmt != 0) {                               // bytes: (x0 - 1) * CI minus its 16-byte floor
+            if (XF == X_RUNTIME ? p.stem_fmt != 0 : x_is_nhwc(XF)) {   // NHWC: (x0 - 1) * CI minus its 16-byte floor
                 int n_, rr_, ty_, tx_;
                 fdivmod(static_cast<uint32_t>(t), p.fd_tpi, n_, rr_);
                 fdivmod(static_cast<uint32_t>(rr_), p.fd_tx, ty_, tx_);
-                sh = ((tx_ * 8 - 1) * CI) & 15;
+                sh = ((tx_ * 8 - 1) * CI) & (XF == X_RUNTIME ? 15 : x_per_16B(XF) - 1);
             }
             mbar_wait(bar_p_full + 8 * slot, ph, 2, p.dbg);
             const uint8_t* pb = s_ring + slot * kStemSlotBytes + (p.stem_fmt != 0 ? sh : 0);
@@ -403,7 +439,19 @@ conv_tc_kernel(const __grid_constant__ ConvParams p) {
                 const int e = r + i * 128;
                 if (e < PE) {
                     const int ci = e / 180, rem = e - ci * 180, py = rem / 10, px = rem - py * 10;
-                    const float v = p.stem_fmt == 0 ? pf[(ci * 18 + py) * FW + px] : s_lut[pb[py * UW + px * CI + ci]];
+                    float v;
+                    if constexpr (XF == X_RUNTIME) {
+                        v = p.stem_fmt == 0 ? pf[(ci * 18 + py) * FW + px] : s_lut[pb[py * UW + px * CI + ci]];
+                    } else {
+                        // the element in its format (box geometry: stem.cuh stem_box_w), widened to fp32 -- exact, so
+                        // from here on the same bits as the fp32 NCHW path on x.float()
+                        constexpr int BW = stem_box_w(XF, CI);
+                        const int i = x_is_nhwc(XF) ? py * BW + sh + px * CI + ci
+                                                    : (ci * 18 + py) * BW + (x_per_16B(XF) - 1) + px;
+                        const uint8_t* box = s_ring + slot * kStemSlotBytes;
+                        if constexpr (x_elem_bytes(XF) == 4) v = reinterpret_cast<const float*>(box)[i];
+                        else v = x_widen16<XF>(reinterpret_cast<const uint16_t*>(box)[i]);
+                    }
                     const uint32_t h2 = pack_bf16x2(v, 0.f);                           // hi in the low half
                     const uint32_t l2 = pack_bf16x2(v - __uint_as_float(h2 << 16), 0.f);
                     p2[e] = __byte_perm(h2, l2, 0x5410);                                // hi | lo << 16
@@ -462,7 +510,13 @@ conv_tc_kernel(const __grid_constant__ ConvParams p) {
                 mbar_wait(bar_p_empty + 8 * slot, ph ^ 1, 1, p.dbg);
                 const uint32_t dst = smem_base + p.off_patch + slot * kStemSlotBytes;
                 // (the innermost start coordinate must sit on a 16-byte boundary, see the im2col producer)
-                if (p.stem_fmt == 0) {                           // fp32 [N][C][H][W]: box 16 x 18 x Cin from x0 - 3
+                if constexpr (XF != X_RUNTIME) {                 // box geometry: stem.cuh stem_box_w
+                    mbar_expect_tx(bar_p_full + 8 * slot, stem_box_bytes(XF, CI));
+                    if (x_is_nhwc(XF))
+                        tma_load_3d(dst, &p.tmA0, bar_p_full + 8 * slot, (x0 * CI) & ~(x_per_16B(XF) - 1), y0, n);
+                    else
+                        tma_load_4d(dst, &p.tmA0, bar_p_full + 8 * slot, x0 - (x_per_16B(XF) - 1), y0, 0, n);
+                } else if (p.stem_fmt == 0) {                           // fp32 [N][C][H][W]: box 16 x 18 x Cin from x0 - 3
                     mbar_expect_tx(bar_p_full + 8 * slot, kBytes32);
                     tma_load_4d(dst, &p.tmA0, bar_p_full + 8 * slot, x0 - 3, y0, 0, n);
                 } else {                                         // uint8 [N][H][W * Cin]: box 48 (32) bytes x 18
@@ -799,7 +853,7 @@ conv_tc_kernel(const __grid_constant__ ConvParams p) {
                     for (int c = 0; c < NC; ++c) {
                         if (c < p.ncls) {
                             const size_t o = ((static_cast<size_t>(n) * p.ncls + c) * p.H + y) * p.W + x;
-                            if (p.logits) p.logits[o] = z[c];
+                            if (p.logits) store_logit<LT>(p.logits, o, z[c]);
                             if (p.mask && !p.mask_bits) p.mask[o] = z[c] > p.thr[c] ? 1 : 0;
                         }
                     }

@@ -7,12 +7,61 @@
 // tensor as it is (fp32 NCHW like inference.py:36-42 produces, or the raw uint8
 // HWC frame, scaled by /255 here) and writes the NHWC bf16 layout every later
 // kernel consumes.
+//
+// Float inputs may also be fp16 / bf16 and NCHW or NHWC (the storage of a channels_last tensor): an element is
+// widened to fp32 where it is read, which is exact for every 16-bit value, so everything after the read sees the
+// same fp32 value as for the fp32 NCHW tensor x.float().contiguous().
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include "ptx.cuh"
 
 namespace ub {
 
-enum : int { X_F32_NCHW = 0, X_U8_NHWC = 1 };
+// input formats (include/unetb200.h UNETB200_X_*); NHWC = [N][H][W][C] in memory
+enum : int { X_F32_NCHW = 0, X_U8_NHWC = 1, X_F16_NCHW = 2, X_BF16_NCHW = 3, X_F32_NHWC = 4, X_F16_NHWC = 5,
+             X_BF16_NHWC = 6 };
+// kernel template argument "format chosen at run time": X_F32_NCHW or X_U8_NHWC by the launch's x_fmt / stem_fmt
+// (the two original formats share one instantiation per kernel; every other format has its own)
+constexpr int X_RUNTIME = -1;
+constexpr int kNumXFormats = 7;
+
+__host__ __device__ constexpr int x_elem_bytes(int f) {
+    return f == X_U8_NHWC ? 1 : ((f == X_F32_NCHW || f == X_F32_NHWC) ? 4 : 2);
+}
+__host__ __device__ constexpr bool x_is_nhwc(int f) { return f == X_U8_NHWC || f >= X_F32_NHWC; }
+__host__ __device__ constexpr int x_per_16B(int f) { return 16 / x_elem_bytes(f); }
+
+// Input box of the tensor-core stem (conv_tc.cuh A_STEM, make_input_map): the 18 x 10 halo patch of a tile is one
+// TMA box, and a TMA tile load faults unless the byte offset of its innermost start coordinate is a multiple of 16.
+//   NCHW: 4-D map (W, H, C, N), box (stem_box_w, 18, C, 1) from column x0 - (x_per_16B - 1): patch columns
+//         x_per_16B - 1 .. x_per_16B + 8 of the box rows
+//   NHWC: 3-D map (W * C, H, N), box (stem_box_w, 18, 1) from the 16-byte floor of x0 * C: the patch starts
+//         sh = (x0 * C) mod x_per_16B elements into each box row
+// with x0 = the tile's first column - 1.  The width is the smallest 16-byte multiple that covers the patch row
+// from any start: fp32 NCHW 16, 16-bit NCHW 24, NHWC (C = 3) fp32 36 / 16-bit 40 / uint8 48 elements.
+__host__ __device__ constexpr int stem_box_w(int f, int cin) {
+    return ((x_is_nhwc(f) ? 10 * cin : 10) + 2 * (x_per_16B(f) - 1)) / x_per_16B(f) * x_per_16B(f);
+}
+__host__ __device__ constexpr int stem_box_bytes(int f, int cin) {
+    return stem_box_w(f, cin) * x_elem_bytes(f) * 18 * (x_is_nhwc(f) ? 1 : cin);
+}
+
+// 16-bit element -> fp32 (exact)
+template <int XF>
+__device__ __forceinline__ float x_widen16(uint16_t u) {
+    if constexpr (XF == X_F16_NCHW || XF == X_F16_NHWC) return __half2float(__ushort_as_half(u));
+    else return __uint_as_float(static_cast<uint32_t>(u) << 16);
+}
+
+// element i of a float-format input in global memory, as fp32
+template <int XF>
+__device__ __forceinline__ float x_load(const void* x, size_t i) {
+    static_assert(XF != X_U8_NHWC && XF != X_RUNTIME, "float formats only");
+    if constexpr (x_elem_bytes(XF) == 4) return __ldg(static_cast<const float*>(x) + i);
+    else return x_widen16<XF>(__ldg(static_cast<const unsigned short*>(x) + i));
+}
 
 struct StemParams {
     const void* x;        // input, format per x_fmt
@@ -25,7 +74,7 @@ struct StemParams {
 
 constexpr int kStemTX = 32, kStemTY = 8;
 
-template <int CIN>
+template <int CIN, int XF = X_RUNTIME>
 __global__ void __launch_bounds__(256) stem_conv_kernel(const StemParams p) {
     __shared__ __align__(16) float s_w[9 * CIN * 64];
     __shared__ __align__(16) float s_b[64];
@@ -45,7 +94,10 @@ __global__ void __launch_bounds__(256) stem_conv_kernel(const StemParams p) {
         const int y = y0 + yy - 1, x = x0 + xx - 1;
         float v = 0.f;
         if (y >= 0 && y < p.H && x >= 0 && x < p.W) {
-            if (p.x_fmt == X_F32_NCHW) {
+            if constexpr (XF != X_RUNTIME) {
+                v = x_load<XF>(p.x, x_is_nhwc(XF) ? ((static_cast<size_t>(n) * p.H + y) * p.W + x) * CIN + ci
+                                                  : ((static_cast<size_t>(n) * CIN + ci) * p.H + y) * p.W + x);
+            } else if (p.x_fmt == X_F32_NCHW) {
                 v = __ldg(static_cast<const float*>(p.x) +
                           ((static_cast<size_t>(n) * CIN + ci) * p.H + y) * p.W + x);
             } else {

@@ -113,33 +113,43 @@ int make_w_map(CUtensorMap* m, const void* base, int cin, int rows, int taps, in
     return 0;
 }
 
-// network input of the first conv (conv_tc.cuh, A_STEM): the 18 x 10 halo patch of a tile as one TMA box.
-//   fp32 [N][C][H][W]      -> 4-D map (W, H, C, N), box (16, 18, C, 1)
-//   uint8 [N][H][W][C]     -> 3-D map (W * C, H, N), box (48 | 32 bytes, 18, 1)
+bool valid_x_fmt(int x_fmt) { return x_fmt >= 0 && x_fmt < ub::kNumXFormats; }
+
+// network input of the first conv (conv_tc.cuh, A_STEM): the 18 x 10 halo patch of a tile as one TMA box
+// (geometry: stem.cuh stem_box_w).
+//   NCHW [N][C][H][W]      -> 4-D map (W, H, C, N), box (16 fp32 | 24 16-bit elements, 18, C, 1)
+//   NHWC [N][H][W][C]      -> 3-D map (W * C, H, N), box (48 | 32 bytes for uint8, 36 | 16 fp32, 40 | 24 16-bit, 18, 1)
 // The boxes are wider than the 10 columns used because a TMA tile load faults unless its innermost start
 // coordinate sits on a 16-byte boundary (conv_tc.cuh).  Out-of-image elements are zero-filled, which is the conv
-// padding (byte 0 -> 0 / 255).
+// padding (byte 0 -> 0 / 255; +0.0 in every float format).
 int make_input_map(CUtensorMap* m, const void* x, int x_fmt, int cin, int W, int H, int N) {
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return fail(UNETB200_ECUDA, "cuTensorMapEncodeTiled entry point unavailable");
+    if (!valid_x_fmt(x_fmt)) return fail(UNETB200_EINVAL, "unknown x_fmt");
     if (reinterpret_cast<uintptr_t>(x) & 15) return fail(UNETB200_EINVAL, "stem: the input tensor must be 16-byte aligned");
+    const uint64_t e = ub::x_elem_bytes(x_fmt);
+    const CUtensorMapDataType dt = e == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
+                                 : e == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8
+                                 : (x_fmt == UNETB200_X_F16_NCHW || x_fmt == UNETB200_X_F16_NHWC) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+                                                                                                  : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    const cuuint32_t bw = static_cast<cuuint32_t>(ub::stem_box_w(x_fmt, cin));
     CUresult r;
-    if (x_fmt == UNETB200_X_F32_NCHW) {
-        if (W % 4) return fail(UNETB200_EINVAL, "stem: float input needs a width that is a multiple of 4");
+    if (!ub::x_is_nhwc(x_fmt)) {
+        if ((W * e) % 16) return fail(UNETB200_EINVAL, "stem: NCHW input needs rows of a multiple of 16 bytes");
         cuuint64_t dims[4] = {uint64_t(W), uint64_t(H), uint64_t(cin), uint64_t(N)};
-        cuuint64_t strides[3] = {uint64_t(W) * 4, uint64_t(H) * W * 4, uint64_t(cin) * H * W * 4};
-        cuuint32_t box[4] = {16, 18, uint32_t(cin), 1};
+        cuuint64_t strides[3] = {uint64_t(W) * e, uint64_t(H) * W * e, uint64_t(cin) * H * W * e};
+        cuuint32_t box[4] = {bw, 18, uint32_t(cin), 1};
         cuuint32_t estr[4] = {1, 1, 1, 1};
-        r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<void*>(x), dims, strides, box, estr,
+        r = enc(m, dt, 4, const_cast<void*>(x), dims, strides, box, estr,
                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     } else {
-        if ((W * cin) % 16) return fail(UNETB200_EINVAL, "stem: uint8 input needs W * channels to be a multiple of 16");
+        if ((W * cin * e) % 16) return fail(UNETB200_EINVAL, "stem: NHWC input needs rows of a multiple of 16 bytes");
         cuuint64_t dims[3] = {uint64_t(W) * cin, uint64_t(H), uint64_t(N)};
-        cuuint64_t strides[2] = {uint64_t(W) * cin, uint64_t(H) * W * cin};
-        cuuint32_t box[3] = {cin == 1 ? 32u : 48u, 18, 1};
+        cuuint64_t strides[2] = {uint64_t(W) * cin * e, uint64_t(H) * W * cin * e};
+        cuuint32_t box[3] = {bw, 18, 1};
         cuuint32_t estr[3] = {1, 1, 1};
-        r = enc(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(x), dims, strides, box, estr,
+        r = enc(m, dt, 3, const_cast<void*>(x), dims, strides, box, estr,
                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     }
@@ -276,10 +286,11 @@ struct ConvLaunch {
     bool phase = false;             // conv_phase_kernel (conv_phase.cuh): up-conv folded into the 3x3 conv
 };
 
-template <int BN, int TAPS, int AMODE, int EPI, int X = 0, bool PAIR = false>
+template <int BN, int TAPS, int AMODE, int EPI, int X = 0, bool PAIR = false, int XF = ub::X_RUNTIME,
+          int LT = ub::LOGITS_F32>
 ConvLaunch conv_inst() {
     ConvLaunch l;
-    l.fn = ub::conv_tc_kernel<BN, TAPS, AMODE, EPI, X, PAIR>;
+    l.fn = ub::conv_tc_kernel<BN, TAPS, AMODE, EPI, X, PAIR, XF, LT>;
     l.a_stage = ub::ConvCfg<BN, TAPS, AMODE, PAIR>::A_STAGE;
     l.b_stage = ub::ConvCfg<BN, TAPS, AMODE, PAIR>::B_STAGE;
     l.b_tap = ub::ConvCfg<BN, TAPS, AMODE, PAIR>::B_TAP;
@@ -323,14 +334,47 @@ ConvLaunch conv3_pick_amode(int amode, int epi) {
     }
 }
 
-template <int CIN>
+// fused head (conv1.net.3 + out_conv): n_classes == 3 (the reference's configuration) has its own instantiation;
+// one per logits element type
+template <int AMODE, bool PAIR>
+ConvLaunch head_inst(int ncls, int logits_type) {
+    const bool three = ncls == 3;
+    switch (logits_type) {
+        case ub::LOGITS_F32:
+            return three ? conv_inst<64, 9, AMODE, ub::EPI_HEAD, 3, PAIR>() : conv_inst<64, 9, AMODE, ub::EPI_HEAD, 0, PAIR>();
+        case ub::LOGITS_F16:
+            return three ? conv_inst<64, 9, AMODE, ub::EPI_HEAD, 3, PAIR, ub::X_RUNTIME, ub::LOGITS_F16>()
+                         : conv_inst<64, 9, AMODE, ub::EPI_HEAD, 0, PAIR, ub::X_RUNTIME, ub::LOGITS_F16>();
+        case ub::LOGITS_BF16:
+            return three ? conv_inst<64, 9, AMODE, ub::EPI_HEAD, 3, PAIR, ub::X_RUNTIME, ub::LOGITS_BF16>()
+                         : conv_inst<64, 9, AMODE, ub::EPI_HEAD, 0, PAIR, ub::X_RUNTIME, ub::LOGITS_BF16>();
+    }
+    return ConvLaunch();
+}
+
+template <int CIN, int XF = ub::X_RUNTIME>
 ConvLaunch stem_inst() {
     ConvLaunch l;
-    l.fn = ub::conv_tc_kernel<64, 1, ub::A_STEM, ub::EPI_STORE, CIN>;
+    l.fn = ub::conv_tc_kernel<64, 1, ub::A_STEM, ub::EPI_STORE, CIN, false, XF>;
     l.a_stage = ub::ConvCfg<64, 1, ub::A_STEM>::A_STAGE;
     l.b_stage = ub::ConvCfg<64, 1, ub::A_STEM>::B_STAGE;
     l.b_tap = ub::ConvCfg<64, 1, ub::A_STEM>::B_TAP;
     return l;
+}
+
+// im2col stem: fp32 NCHW and uint8 NHWC share the run-time-format instantiation; every other format has its own
+template <int CIN>
+ConvLaunch stem_pick_fmt(int x_fmt) {
+    switch (x_fmt) {
+        case UNETB200_X_F32_NCHW:
+        case UNETB200_X_U8_NHWC: return stem_inst<CIN>();
+        case UNETB200_X_F16_NCHW: return stem_inst<CIN, ub::X_F16_NCHW>();
+        case UNETB200_X_BF16_NCHW: return stem_inst<CIN, ub::X_BF16_NCHW>();
+        case UNETB200_X_F32_NHWC: return stem_inst<CIN, ub::X_F32_NHWC>();
+        case UNETB200_X_F16_NHWC: return stem_inst<CIN, ub::X_F16_NHWC>();
+        case UNETB200_X_BF16_NHWC: return stem_inst<CIN, ub::X_BF16_NHWC>();
+    }
+    return ConvLaunch();
 }
 
 #ifdef UNETB200_TEST_VARIANTS
@@ -345,7 +389,8 @@ ConvLaunch stemp_inst() {
 }
 #endif
 
-ConvLaunch pick_conv(int taps, int bn, int amode, int epi, int stem_cin = 0, int ncls = 0, bool pair = false) {
+ConvLaunch pick_conv(int taps, int bn, int amode, int epi, int stem_cin = 0, int ncls = 0, bool pair = false,
+                     int stem_fmt = UNETB200_X_F32_NCHW, int logits_type = ub::LOGITS_F32) {
     if (amode == ub::A_STEMP) {
 #ifdef UNETB200_TEST_VARIANTS
         switch (stem_cin) {
@@ -357,9 +402,7 @@ ConvLaunch pick_conv(int taps, int bn, int amode, int epi, int stem_cin = 0, int
         return ConvLaunch();
     }
     if (pair && amode != ub::A_STEM && amode != ub::A_STEMP && (taps == 1 || amode == ub::A_HALO)) {
-        if (epi == ub::EPI_HEAD)
-            return ncls == 3 ? conv_inst<64, 9, ub::A_HALO, ub::EPI_HEAD, 3, true>()
-                             : conv_inst<64, 9, ub::A_HALO, ub::EPI_HEAD, 0, true>();
+        if (epi == ub::EPI_HEAD) return head_inst<ub::A_HALO, true>(ncls, logits_type);
         switch (bn) {
             case 64: return pair_pick<64>(taps, epi);
             case 128: return pair_pick<128>(taps, epi);
@@ -369,8 +412,8 @@ ConvLaunch pick_conv(int taps, int bn, int amode, int epi, int stem_cin = 0, int
     }
     if (amode == ub::A_STEM) {
         switch (stem_cin) {
-            case 1: return stem_inst<1>();
-            case 3: return stem_inst<3>();
+            case 1: return stem_pick_fmt<1>(stem_fmt);
+            case 3: return stem_pick_fmt<3>(stem_fmt);
         }
         return ConvLaunch();
     }
@@ -383,14 +426,12 @@ ConvLaunch pick_conv(int taps, int bn, int amode, int epi, int stem_cin = 0, int
         return ConvLaunch();
     }
     if (epi == ub::EPI_HEAD) {
-        // n_classes == 3 (the reference's configuration) has its own instantiation
-        const bool three = ncls == 3;
         switch (amode) {
-            case ub::A_TAP: return three ? conv_inst<64, 9, ub::A_TAP, ub::EPI_HEAD, 3>() : conv_inst<64, 9, ub::A_TAP, ub::EPI_HEAD>();
+            case ub::A_TAP: return head_inst<ub::A_TAP, false>(ncls, logits_type);
 #ifdef UNETB200_TEST_VARIANTS
-            case ub::A_COL3: return three ? conv_inst<64, 9, ub::A_COL3, ub::EPI_HEAD, 3>() : conv_inst<64, 9, ub::A_COL3, ub::EPI_HEAD>();
+            case ub::A_COL3: return head_inst<ub::A_COL3, false>(ncls, logits_type);
 #endif
-            case ub::A_HALO: return three ? conv_inst<64, 9, ub::A_HALO, ub::EPI_HEAD, 3>() : conv_inst<64, 9, ub::A_HALO, ub::EPI_HEAD>();
+            case ub::A_HALO: return head_inst<ub::A_HALO, false>(ncls, logits_type);
         }
         return ConvLaunch();
     }
@@ -402,8 +443,11 @@ ConvLaunch pick_conv(int taps, int bn, int amode, int epi, int stem_cin = 0, int
     return ConvLaunch();
 }
 
+typedef void (*StemKernel)(const ub::StemParams);
+
 struct Step {
     int kind = 0;              // 0 = stem, 1 = conv_tc
+    StemKernel stem_fn = nullptr;   // kind 0: the CUDA-core stem instantiation (stem.cuh)
     int layer = -1;            // index into the layer table (profiling)
     ConvLaunch conv;
     ub::ConvParams cp;
@@ -429,7 +473,8 @@ struct ConvDesc {
     const float* head_w = nullptr;
     const float* head_b = nullptr;
     int ncls = 0;
-    float* logits = nullptr;
+    void* logits = nullptr;
+    int logits_type = ub::LOGITS_F32;   // element type of `logits` (UNETB200_LOGITS_*)
     uint8_t* mask = nullptr;
     int mask_bits = 0;          // 1 = mask is bit-packed [N][ncls][H][W/8]
     int bn = 128, amode = ub::A_COL3;
@@ -510,7 +555,18 @@ int build_row_step(const ConvDesc& d, int num_sms, Step* st) {
     switch (d.epi) {
         case ub::EPI_STORE: cl.fn = ub::conv_row_kernel<ub::EPI_STORE>; break;
         case ub::EPI_STORE_POOL: cl.fn = ub::conv_row_kernel<ub::EPI_STORE_POOL>; break;
-        case ub::EPI_HEAD: cl.fn = d.ncls == 3 ? ub::conv_row_kernel<ub::EPI_HEAD, 3> : ub::conv_row_kernel<ub::EPI_HEAD, 0>; break;
+        case ub::EPI_HEAD:
+            switch (d.logits_type) {
+                case ub::LOGITS_F32: cl.fn = d.ncls == 3 ? ub::conv_row_kernel<ub::EPI_HEAD, 3> : ub::conv_row_kernel<ub::EPI_HEAD, 0>; break;
+                case ub::LOGITS_F16:
+                    cl.fn = d.ncls == 3 ? ub::conv_row_kernel<ub::EPI_HEAD, 3, ub::LOGITS_F16> : ub::conv_row_kernel<ub::EPI_HEAD, 0, ub::LOGITS_F16>;
+                    break;
+                case ub::LOGITS_BF16:
+                    cl.fn = d.ncls == 3 ? ub::conv_row_kernel<ub::EPI_HEAD, 3, ub::LOGITS_BF16> : ub::conv_row_kernel<ub::EPI_HEAD, 0, ub::LOGITS_BF16>;
+                    break;
+                default: return fail(UNETB200_EINVAL, "unknown logits_type");
+            }
+            break;
         default: return fail(UNETB200_EINVAL, "row kernel: unsupported epilogue");
     }
     ub::ConvParams& p = st->cp;
@@ -766,7 +822,18 @@ int build_ps64_step(const ConvDesc& d, int num_sms, Step* st) {
     switch (d.epi) {
         case ub::EPI_STORE: cl.fn = ub::conv_ps64_kernel<ub::EPI_STORE>; break;
         case ub::EPI_STORE_POOL: cl.fn = ub::conv_ps64_kernel<ub::EPI_STORE_POOL>; break;
-        case ub::EPI_HEAD: cl.fn = d.ncls == 3 ? ub::conv_ps64_kernel<ub::EPI_HEAD, 3> : ub::conv_ps64_kernel<ub::EPI_HEAD, 0>; break;
+        case ub::EPI_HEAD:
+            switch (d.logits_type) {
+                case ub::LOGITS_F32: cl.fn = d.ncls == 3 ? ub::conv_ps64_kernel<ub::EPI_HEAD, 3> : ub::conv_ps64_kernel<ub::EPI_HEAD, 0>; break;
+                case ub::LOGITS_F16:
+                    cl.fn = d.ncls == 3 ? ub::conv_ps64_kernel<ub::EPI_HEAD, 3, ub::LOGITS_F16> : ub::conv_ps64_kernel<ub::EPI_HEAD, 0, ub::LOGITS_F16>;
+                    break;
+                case ub::LOGITS_BF16:
+                    cl.fn = d.ncls == 3 ? ub::conv_ps64_kernel<ub::EPI_HEAD, 3, ub::LOGITS_BF16> : ub::conv_ps64_kernel<ub::EPI_HEAD, 0, ub::LOGITS_BF16>;
+                    break;
+                default: return fail(UNETB200_EINVAL, "unknown logits_type");
+            }
+            break;
         default: return fail(UNETB200_EINVAL, "phase-stacked kernel: unsupported epilogue");
     }
     ub::ConvParams& p = st->cp;
@@ -888,7 +955,10 @@ int build_conv_step(const ConvDesc& d, int num_sms, Step* st) {
     if (d.epi == ub::EPI_HEAD && d.cout != 64)
         return fail(UNETB200_EINVAL, "fused head needs cout == 64");
     st->kind = 1;
-    st->conv = pick_conv(d.taps, bn, d.amode, d.epi, d.stem_cin, d.ncls, d.pair != 0);
+    if (d.logits_type != ub::LOGITS_F32 && !(d.epi == ub::EPI_HEAD &&
+                                             (d.logits_type == ub::LOGITS_F16 || d.logits_type == ub::LOGITS_BF16)))
+        return fail(UNETB200_EINVAL, "unknown logits_type");
+    st->conv = pick_conv(d.taps, bn, d.amode, d.epi, d.stem_cin, d.ncls, d.pair != 0, d.stem_fmt, d.logits_type);
     if (!st->conv.fn)
         return fail(UNETB200_EINVAL, "conv: no kernel for this configuration (A_COL3 and the patch stem exist only in "
                                      "builds with -DUNETB200_TEST_VARIANTS)");
@@ -1037,21 +1107,39 @@ int launch_step(Step& st, cudaStream_t stream) {
         cfg.numAttrs = na;
         UB_CUDA(cudaLaunchKernelEx(&cfg, st.conv.fn, st.cp));
     } else {
-        switch (st.stem_cin) {
-            case 1: ub::stem_conv_kernel<1><<<st.grid, st.block, 0, stream>>>(st.sp); break;
-            case 3: ub::stem_conv_kernel<3><<<st.grid, st.block, 0, stream>>>(st.sp); break;
-            case 4: ub::stem_conv_kernel<4><<<st.grid, st.block, 0, stream>>>(st.sp); break;
-            default: return fail(UNETB200_EINVAL, "stem: n_channels must be 1, 3 or 4");
-        }
+        if (!st.stem_fn) return fail(UNETB200_EINVAL, "stem: no kernel for this configuration");
+        st.stem_fn<<<st.grid, st.block, 0, stream>>>(st.sp);
     }
     UB_CUDA(cudaGetLastError());
     return 0;
 }
 
+// CUDA-core stem: fp32 NCHW and uint8 NHWC share the run-time-format instantiation; every other format has its own
+template <int CIN>
+StemKernel stem_cc_pick_fmt(int x_fmt) {
+    switch (x_fmt) {
+        case UNETB200_X_F32_NCHW:
+        case UNETB200_X_U8_NHWC: return ub::stem_conv_kernel<CIN>;
+        case UNETB200_X_F16_NCHW: return ub::stem_conv_kernel<CIN, ub::X_F16_NCHW>;
+        case UNETB200_X_BF16_NCHW: return ub::stem_conv_kernel<CIN, ub::X_BF16_NCHW>;
+        case UNETB200_X_F32_NHWC: return ub::stem_conv_kernel<CIN, ub::X_F32_NHWC>;
+        case UNETB200_X_F16_NHWC: return ub::stem_conv_kernel<CIN, ub::X_F16_NHWC>;
+        case UNETB200_X_BF16_NHWC: return ub::stem_conv_kernel<CIN, ub::X_BF16_NHWC>;
+    }
+    return nullptr;
+}
+
 int build_stem_step(const void* x, int x_fmt, int cin, const float* w, const float* bias, int n,
                     int h, int wd, void* out, Step* st) {
-    if (x_fmt != UNETB200_X_F32_NCHW && x_fmt != UNETB200_X_U8_NHWC)
-        return fail(UNETB200_EINVAL, "unknown x_fmt");
+    if (!valid_x_fmt(x_fmt)) return fail(UNETB200_EINVAL, "unknown x_fmt");
+    switch (cin) {
+        case 1: st->stem_fn = stem_cc_pick_fmt<1>(x_fmt); break;
+        case 3: st->stem_fn = stem_cc_pick_fmt<3>(x_fmt); break;
+        case 4: st->stem_fn = stem_cc_pick_fmt<4>(x_fmt); break;
+        default: return fail(UNETB200_EINVAL, "stem: n_channels must be 1, 3 or 4");
+    }
+    if (reinterpret_cast<uintptr_t>(x) % ub::x_elem_bytes(x_fmt))
+        return fail(UNETB200_EINVAL, "stem: the input tensor is not aligned to its element size");
     st->kind = 0;
     st->stem_cin = cin;
     st->sp.x = x;
@@ -1072,8 +1160,10 @@ int build_stem_step(const void* x, int x_fmt, int cin, const float* w, const flo
 // user's tensor, hi/lo-split bf16 GEMM over two K slices against the [64][128] packed weights.
 int build_stem_tc_step(const void* x, int x_fmt, int cin, const void* w_tc, const float* bias, int n,
                        int h, int wd, void* out, int num_sms, int* dbg, Step* st, bool patch = false) {
-    if (x_fmt != UNETB200_X_F32_NCHW && x_fmt != UNETB200_X_U8_NHWC)
-        return fail(UNETB200_EINVAL, "unknown x_fmt");
+    if (!valid_x_fmt(x_fmt)) return fail(UNETB200_EINVAL, "unknown x_fmt");
+    if (patch && x_fmt != UNETB200_X_F32_NCHW && x_fmt != UNETB200_X_U8_NHWC)
+        return fail(UNETB200_EINVAL, "patch stem (stem_tc = 2): fp32 NCHW and uint8 NHWC inputs only; the fp16 / bf16 and "
+                                     "NHWC float formats run on stem_tc = 0 or 1");
     if (patch ? !(cin == 1 || cin == 3 || cin == 4) : !(cin == 1 || cin == 3))
         return fail(UNETB200_EINVAL, "tensor-core stem: unsupported n_channels");
     ConvDesc d;
@@ -1101,7 +1191,8 @@ int check_sm100() {
     return 0;
 }
 
-typedef std::tuple<const void*, int, int, int, int, void*, float*, uint8_t*, int> PlanKey;
+// (x, x_fmt, n, H, W, workspace, logits, logits_type, mask, mask_bits): everything baked into a plan's launches
+typedef std::tuple<const void*, int, int, int, int, void*, void*, int, uint8_t*, int> PlanKey;
 
 struct Plan {
     std::vector<Step> steps;
@@ -1193,7 +1284,7 @@ WsLayout ws_layout(int n, int h, int w, int bw) {
 }
 
 int build_plan(unetb200_handle_t h, const void* x, int x_fmt, int n, int H, int W, void* ws,
-               float* logits, uint8_t* mask, int mask_bits, Plan* plan) {
+               void* logits, int logits_type, uint8_t* mask, int mask_bits, Plan* plan) {
     const int bw = h->arch.base_width;
     const WsLayout L = ws_layout(n, H, W, bw);
     char* base = static_cast<char*>(ws);
@@ -1295,7 +1386,7 @@ int build_plan(unetb200_handle_t h, const void* x, int x_fmt, int n, int H, int 
             d.w = Wp(21); d.bias = Bp(21);
             d.n = n; d.h = H; d.wd = W; d.cout = bw; d.relu = 1; d.taps = 9; d.epi = ub::EPI_HEAD;
             d.head_w = reinterpret_cast<const float*>(Wp(22)); d.head_b = Bp(22);
-            d.ncls = h->arch.n_classes; d.logits = logits; d.mask = mask; d.mask_bits = mask_bits;
+            d.ncls = h->arch.n_classes; d.logits = logits; d.logits_type = logits_type; d.mask = mask; d.mask_bits = mask_bits;
             d.bn = 64; d.amode = (h->ps64 & 2) ? ub::A_PS64 : ((h->row64 & 1) ? ub::A_ROW : h->amode); d.wstat = h->wstat; d.pf_items = h->pf_items; d.epi2 = h->epi2; d.min_na = h->min_na; d.pair = h->pair >= 1; d.dbg = h->dbg;
             Step st;
             if ((rc = build_conv_step(d, h->num_sms, &st))) return rc;
@@ -1600,8 +1691,8 @@ uint64_t unetb200_workspace_bytes(unetb200_handle_t h, int n, int height, int wi
 }
 
 static int forward_impl(unetb200_handle_t h, const void* x, int x_fmt, int n, int height, int width,
-                        void* workspace, uint64_t workspace_bytes, float* logits, uint8_t* mask, int mask_bits,
-                        const float* logit_thr, void* stream) {
+                        void* workspace, uint64_t workspace_bytes, void* logits, int logits_type, uint8_t* mask,
+                        int mask_bits, const float* logit_thr, void* stream) {
     if (!h) return fail(UNETB200_EINVAL, "handle is NULL");
     if (!x || !workspace) return fail(UNETB200_EINVAL, "x/workspace pointer is NULL");
     if (n <= 0 || height <= 0 || width <= 0) return fail(UNETB200_EINVAL, "empty input");
@@ -1610,6 +1701,9 @@ static int forward_impl(unetb200_handle_t h, const void* x, int x_fmt, int n, in
                     "H and W must be divisible by 16 (the reference fails in torch.cat otherwise), got " +
                         std::to_string(height) + "x" + std::to_string(width));
     if (!logits && !mask) return fail(UNETB200_EINVAL, "both outputs are NULL");
+    if (!valid_x_fmt(x_fmt)) return fail(UNETB200_EINVAL, "unknown x_fmt");
+    if (!(logits_type == UNETB200_LOGITS_F32 || logits_type == UNETB200_LOGITS_F16 || logits_type == UNETB200_LOGITS_BF16))
+        return fail(UNETB200_EINVAL, "unknown logits_type");
     if (mask && !logit_thr) return fail(UNETB200_EINVAL, "mask requested without thresholds");
     const uint64_t need = ws_layout(n, height, width, h->arch.base_width).total;
     if (workspace_bytes < need)
@@ -1638,11 +1732,11 @@ static int forward_impl(unetb200_handle_t h, const void* x, int x_fmt, int n, in
         UB_CUDA(cudaSetDevice(h->device));
         guard.switched = true;
     }
-    PlanKey key(x, x_fmt, n, height, width, workspace, logits, mask, mask_bits);
+    PlanKey key(x, x_fmt, n, height, width, workspace, logits, logits_type, mask, mask_bits);
     auto it = h->plans.find(key);
     if (it == h->plans.end()) {
         Plan plan;
-        int rc = build_plan(h, x, x_fmt, n, height, width, workspace, logits, mask, mask_bits, &plan);
+        int rc = build_plan(h, x, x_fmt, n, height, width, workspace, logits, logits_type, mask, mask_bits, &plan);
         if (rc) return rc;
         if (h->plans.size() > 64) destroy_plans(h->plans);
         it = h->plans.emplace(key, std::move(plan)).first;
@@ -1716,14 +1810,22 @@ static int forward_impl(unetb200_handle_t h, const void* x, int x_fmt, int n, in
 int unetb200_forward(unetb200_handle_t h, const void* x, int x_fmt, int n, int height, int width,
                      void* workspace, uint64_t workspace_bytes, float* logits, uint8_t* mask,
                      const float* logit_thr, void* stream) {
-    return forward_impl(h, x, x_fmt, n, height, width, workspace, workspace_bytes, logits, mask, 0, logit_thr, stream);
+    return forward_impl(h, x, x_fmt, n, height, width, workspace, workspace_bytes, logits, UNETB200_LOGITS_F32, mask, 0,
+                        logit_thr, stream);
 }
 
 int unetb200_forward_bits(unetb200_handle_t h, const void* x, int x_fmt, int n, int height, int width,
                           void* workspace, uint64_t workspace_bytes, float* logits, uint8_t* mask_bits,
                           const float* logit_thr, void* stream) {
-    return forward_impl(h, x, x_fmt, n, height, width, workspace, workspace_bytes, logits, mask_bits, 1, logit_thr,
-                        stream);
+    return forward_impl(h, x, x_fmt, n, height, width, workspace, workspace_bytes, logits, UNETB200_LOGITS_F32,
+                        mask_bits, 1, logit_thr, stream);
+}
+
+int unetb200_forward_typed(unetb200_handle_t h, const void* x, int x_fmt, int n, int height, int width,
+                           void* workspace, uint64_t workspace_bytes, void* logits, int logits_type,
+                           uint8_t* mask, int mask_bits, const float* logit_thr, void* stream) {
+    return forward_impl(h, x, x_fmt, n, height, width, workspace, workspace_bytes, logits, logits_type, mask,
+                        mask_bits ? 1 : 0, logit_thr, stream);
 }
 
 int unetb200_layer_times(unetb200_handle_t h, float* ms, int count) {
@@ -1779,10 +1881,12 @@ int unetb200_conv3x3(const void* src0, int c0, const void* src1, int c1, const v
 
 int unetb200_conv3x3_head(const void* src0, int c0, const void* w_packed, const float* bias,
                           const float* head_w, const float* head_b, int n_classes, int n, int height,
-                          int width, float* logits, uint8_t* mask, const float* logit_thr, int amode,
+                          int width, void* logits, uint8_t* mask, const float* logit_thr, int amode,
                           int wstat, void* stream) {
     int rc;
     if ((rc = check_sm100())) return rc;
+    const int logits_type = (wstat >> 3) & 3;
+    if (logits_type == 3) return fail(UNETB200_EINVAL, "unknown logits_type (wstat bits 3-4)");
     if (!src0 || !w_packed || !bias || !head_w || !head_b) return fail(UNETB200_EINVAL, "NULL pointer");
     if (n_classes < 1 || n_classes > ub::kMaxClasses) return fail(UNETB200_EINVAL, "n_classes must be in 1..8");
     if (mask && !logit_thr) return fail(UNETB200_EINVAL, "mask requested without thresholds");
@@ -1790,7 +1894,8 @@ int unetb200_conv3x3_head(const void* src0, int c0, const void* w_packed, const 
     d.src0 = src0; d.c0 = c0; d.w = w_packed; d.bias = bias; d.n = n; d.h = height; d.wd = width;
     d.cout = 64; d.relu = 1; d.taps = 9; d.epi = ub::EPI_HEAD; d.head_w = head_w; d.head_b = head_b;
     d.ncls = n_classes; d.logits = logits; d.mask = mask; d.bn = 64; d.amode = amode;
-    d.wstat = wstat & 1; d.pair = (wstat >> 1) & 1; d.mask_bits = (wstat >> 2) & 1; d.dbg = g_hook_dbg();
+    d.wstat = wstat & 1; d.pair = (wstat >> 1) & 1; d.mask_bits = (wstat >> 2) & 1; d.logits_type = logits_type;
+    d.dbg = g_hook_dbg();
     int sms = 0;
     if ((rc = device_num_sms(&sms))) return rc;
     Step st;

@@ -40,6 +40,36 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
 
+# float input dtype -> (NCHW format, NHWC format) of the C ABI (include/unetb200.h UNETB200_X_*)
+_FLOAT_FORMATS = {
+    torch.float32: (nat.X_F32_NCHW, nat.X_F32_NHWC),
+    torch.float16: (nat.X_F16_NCHW, nat.X_F16_NHWC),
+    torch.bfloat16: (nat.X_BF16_NCHW, nat.X_BF16_NHWC),
+}
+# logits dtype -> UNETB200_LOGITS_*
+LOGITS_TYPES = {torch.float32: nat.LOGITS_F32, torch.float16: nat.LOGITS_F16, torch.bfloat16: nat.LOGITS_BF16}
+
+
+def input_format(x: torch.Tensor):
+    """``(fmt, x_for_kernel)``: the C-ABI input format of ``x`` and the tensor whose storage the forward reads.
+
+    uint8 is ``[N,H,W,C]`` raw pixels (``X_U8_NHWC``).  float32 / float16 / bfloat16 are ``[N,C,H,W]``: NCHW when
+    ``x`` is contiguous (also when it is channels-last contiguous as well, as with C = 1 or H = W = 1); NHWC, read in
+    place with no copy, when ``x`` is channels-last contiguous (``x.to(memory_format=torch.channels_last)``);
+    otherwise ``x.contiguous()`` as NCHW.  Every other dtype raises ``RuntimeError``."""
+    if x.dtype == torch.uint8:
+        return nat.X_U8_NHWC, x.contiguous()
+    fmts = _FLOAT_FORMATS.get(x.dtype)
+    if fmts is None:
+        raise RuntimeError(f"input dtype must be float32, float16, bfloat16 ([N,C,H,W]) or uint8 ([N,H,W,C]), "
+                           f"got {x.dtype}")
+    if x.is_contiguous():
+        return fmts[0], x
+    if x.dim() == 4 and x.is_contiguous(memory_format=torch.channels_last):
+        return fmts[1], x
+    return fmts[0], x.contiguous()
+
+
 class Engine:
     """One packed model replica on one GPU."""
 
@@ -150,38 +180,42 @@ class Engine:
     def run(self, x: torch.Tensor, *, want_logits: bool = True,
             thresholds: Optional[Sequence[float]] = None,
             logits_out: Optional[torch.Tensor] = None, mask_out: Optional[torch.Tensor] = None,
-            mask_bits: bool = False):
+            mask_bits: bool = False, logits_dtype: Optional[torch.dtype] = None):
         """Enqueue one forward on the current stream.
 
-        ``x``: float32 ``[N,C,H,W]`` (values as ``inference.preprocess`` makes them) or uint8
-        ``[N,H,W,C]`` raw pixels.  Returns ``(logits | None, mask | None)``; ``mask`` is uint8
-        ``[N,n_classes,H,W]`` with 1 where ``sigmoid(logit) > thresholds[c]``, or, with ``mask_bits``,
-        the same booleans packed eight to a byte: uint8 ``[N,n_classes,H,W/8]``, pixel ``x`` = bit ``x & 7``
-        (LSB first) of byte ``x >> 3`` (:func:`unpack_mask_bits` / ``np.unpackbits(bitorder="little")``).
+        ``x``: float32 / float16 / bfloat16 ``[N,C,H,W]`` (values as ``inference.preprocess`` makes them),
+        contiguous or channels-last (read in place), or uint8 ``[N,H,W,C]`` raw pixels (:func:`input_format`).
+        A 16-bit input gives the same results as ``x.float()``.  Returns ``(logits | None, mask | None)``;
+        ``logits`` is ``[N,n_classes,H,W]`` NCHW-contiguous of ``logits_dtype`` (float32, float16 or bfloat16;
+        default: the dtype of a float input, float32 for uint8), 16-bit logits being the float32 logits rounded to
+        nearest-even.  ``mask`` is uint8 ``[N,n_classes,H,W]`` with 1 where ``sigmoid(logit) > thresholds[c]``
+        (decided on the float32 logits), or, with ``mask_bits``, the same booleans packed eight to a byte: uint8
+        ``[N,n_classes,H,W/8]``, pixel ``x`` = bit ``x & 7`` (LSB first) of byte ``x >> 3``
+        (:func:`unpack_mask_bits` / ``np.unpackbits(bitorder="little")``).
         """
         if x.device != self.device:
             raise RuntimeError(f"input is on {x.device}, engine is on {self.device}")
         if x.dim() != 4:
             raise RuntimeError(f"expected a 4-D input, got shape {tuple(x.shape)}")
-        if x.dtype == torch.float32:
-            fmt = nat.X_F32_NCHW
-            n, c, h, w = x.shape
-        elif x.dtype == torch.uint8:
-            fmt = nat.X_U8_NHWC
+        fmt, x = input_format(x)
+        if fmt == nat.X_U8_NHWC:
             n, h, w, c = x.shape
         else:
-            raise RuntimeError(f"input dtype must be float32 (NCHW) or uint8 (NHWC), got {x.dtype}")
+            n, c, h, w = x.shape
+        if logits_dtype is None:
+            logits_dtype = torch.float32 if x.dtype == torch.uint8 else x.dtype
+        if logits_dtype not in LOGITS_TYPES:
+            raise RuntimeError(f"logits_dtype must be torch.float32, torch.float16 or torch.bfloat16, got {logits_dtype}")
         if c != self.n_channels:
             raise RuntimeError(f"expected {self.n_channels} input channels, got {c}")
         if h % 16 or w % 16:
             # the reference raises RuntimeError from torch.cat for such sizes (unet_model.py:71)
             raise RuntimeError(f"H and W must be divisible by 16, got {h}x{w}")
-        x = x.contiguous()
         thr = None
         out_shape = (n, self.n_classes, h, w)
         mask_shape = (n, self.n_classes, h, w // 8) if mask_bits else out_shape
         if logits_out is not None:
-            self._check_out(logits_out, "logits_out", out_shape, torch.float32)
+            self._check_out(logits_out, "logits_out", out_shape, logits_dtype)
         if mask_out is not None:
             self._check_out(mask_out, "mask_out", mask_shape, torch.uint8)
         with self._lock, torch.cuda.device(self.device):
@@ -190,7 +224,7 @@ class Engine:
             logits = None
             if want_logits:
                 logits = logits_out if logits_out is not None else torch.empty(
-                    out_shape, dtype=torch.float32, device=self.device)
+                    out_shape, dtype=logits_dtype, device=self.device)
             mask = None
             if thresholds is not None:
                 if len(thresholds) != self.n_classes:
@@ -198,10 +232,9 @@ class Engine:
                 thr = (C.c_float * self.n_classes)(*logit_thresholds(thresholds))
                 mask = mask_out if mask_out is not None else torch.empty(
                     mask_shape, dtype=torch.uint8, device=self.device)
-            fwd = self._lib.unetb200_forward_bits if mask_bits else self._lib.unetb200_forward
-            nat.check(fwd(
+            nat.check(self._lib.unetb200_forward_typed(
                 self._handle, x.data_ptr(), fmt, n, h, w, ws_ptr, ws_bytes,
-                _ptr(logits), _ptr(mask), thr, stream))
+                _ptr(logits), LOGITS_TYPES[logits_dtype], _ptr(mask), 1 if mask_bits else 0, thr, stream))
         return logits, mask
 
     def layer_times_ms(self) -> list[float]:

@@ -10,8 +10,12 @@ What changed is where the arithmetic runs.  In eval mode ``UNet.forward`` does
 not execute any ``torch.nn`` op: it hands the input to the sm_100a CUDA library
 (``engine.Engine`` -> ``libunetb200.so``), which runs the 23 layers as
 hand-written tcgen05/TMA kernels with BatchNorm folded into the weights, and
-returns float32 NCHW logits on the same device, exactly like the reference.
-Eval mode has no CPU path: a CPU tensor raises.
+returns NCHW logits on the same device, like the reference.  It accepts float32,
+float16 and bfloat16 inputs, contiguous or channels-last, and returns logits in
+the input's dtype (``m.half().eval(); m(x.half())`` gives float16 logits): a 16-bit
+input is widened exactly to float32 where it is read, the network computes in
+bf16 / fp32 as for float32 input, and 16-bit logits are the float32 logits
+rounded to nearest-even.  Eval mode has no CPU path: a CPU tensor raises.
 
 Training mode (``train.py:103,137`` instantiates this same class) still runs the
 ``torch.nn`` graph -- batch statistics and autograd are not part of the
@@ -124,8 +128,8 @@ class UNet(nn.Module):
             raise RuntimeError(
                 "tw_invoice_unet_ocr_llm_b200.UNet runs its eval forward on a B200 (sm_100a) GPU only; "
                 "got a CPU tensor and there is no CPU path")
-        if x.dtype != torch.float32:
-            raise RuntimeError(f"expected a float32 input like the reference, got {x.dtype}")
+        if x.dtype not in (torch.float32, torch.float16, torch.bfloat16):
+            raise RuntimeError(f"expected a float32, float16 or bfloat16 input, got {x.dtype}")
         logits, _ = self.engine(x.device).run(x, want_logits=True)
         return logits
 
