@@ -242,6 +242,25 @@ int unetb200_resize_bicubic_u8_ps(const uint8_t* src, int n, int h, int w, int c
 int unetb200_mask_bbox(const uint8_t* mask, int n_planes, int h, int w, int32_t* out, void* stream);
 /* Same reduction over bit-packed planes (unetb200_forward_bits): bits uint8 [n_planes, h, w/8], w % 32 == 0. */
 int unetb200_mask_bbox_bits(const uint8_t* bits, int n_planes, int h, int w, int32_t* out, void* stream);
+/* Connected components of binary planes: the regions of each field mask, where unetb200_mask_bbox gives the box of
+ * all set pixels.  mask = byte planes uint8 [n_planes, h, w] (non-zero = set; packed = 0) or bit-packed planes
+ * uint8 [n_planes, h, w/8] in the format of unetb200_forward_bits (packed = 1; w % 32 == 0, 4-byte aligned);
+ * h, w >= 1, h * w < 2^31; connectivity 4 or 8.
+ *   labels     nullable; int32 [n_planes, h, w]: 0 = background, components numbered 1..n in raster order of their
+ *              first pixel -- exactly scipy.ndimage.label with generate_binary_structure(2, 1) (4) / ones((3, 3)) (8)
+ *   comps      int32 [n_planes, max_components, 6] = {xmin, xmax, ymin, ymax, count, label} of the max_components
+ *              (1..16) largest components, count descending then label ascending; extents inclusive as
+ *              unetb200_mask_bbox; unused rows {w, -1, h, -1, 0, 0}
+ *   n_comps    int32 [n_planes]: number of components of each plane (may exceed max_components)
+ *   workspace  device scratch of >= unetb200_components_workspace_bytes(n_planes, h, w) bytes, 16-byte aligned,
+ *              no initialisation needed; at most 14.2 bytes per pixel plus 20 bytes per plane
+ * Outputs are deterministic bits.  Asynchronous: enqueued on `stream`, nothing is allocated.  A null pointer, a bad
+ * size, connectivity or max_components, or a misaligned pointer (int32 arrays 4-byte aligned) is UNETB200_EINVAL;
+ * a short workspace UNETB200_ENOMEM.  The query returns 0 for a bad size. */
+uint64_t unetb200_components_workspace_bytes(int n_planes, int h, int w);
+int unetb200_mask_components(const uint8_t* mask, int packed, int n_planes, int h, int w, int connectivity,
+                             int max_components, int32_t* labels, int32_t* comps, int32_t* n_comps, void* workspace,
+                             uint64_t workspace_bytes, void* stream);
 /* Byte sums of n_boxes (<= 16) rectangles {x1, y1, x2, y2} (half-open, host array of 4*n_boxes ints) of one
  * uint8 [h][w][c] device frame -> sums_dev uint64 [n_boxes] (zeroed here): the `np.array(crop).mean() < 3`
  * rejection of inference.py:121-125 as the exact integer test sum < 3 * (x2-x1)*(y2-y1)*c. */

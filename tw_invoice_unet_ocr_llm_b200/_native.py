@@ -90,6 +90,8 @@ SYMBOLS = {
     "unetb200_resize_bicubic_u8_ps": (_I, [_VP, _I, _I, _I, _I, _I, _VP, _VP, _I, _VP, _VP, _I, _VP, _VP, _I, _I, _VP]),
     "unetb200_mask_bbox": (_I, [_VP, _I, _I, _I, _VP, _VP]),
     "unetb200_mask_bbox_bits": (_I, [_VP, _I, _I, _I, _VP, _VP]),
+    "unetb200_components_workspace_bytes": (_U64, [_I, _I, _I]),
+    "unetb200_mask_components": (_I, [_VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _U64, _VP]),
     "unetb200_box_sums": (_I, [_VP, _I, _I, _I, C.POINTER(C.c_int32), _I, _VP, _VP]),
     "unetb200_box_sums_ps": (_I, [_VP, _I, _I, _I, _I, C.POINTER(C.c_int32), _I, _VP, _VP]),
     "unetb200_test_fastdiv": (C.c_uint32, [C.c_uint32, C.c_uint32]),

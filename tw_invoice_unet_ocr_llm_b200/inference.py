@@ -16,6 +16,8 @@ keeps working unmodified.  Differences, all internal:
   too (``prepost.mask_bbox``); other PIL modes take the reference's PIL calls on the host.
 * ``run_unet_batch`` (new, additive) does the same for a list of images in one
   batched forward.
+* ``run_unet_instances`` (new, additive) returns one crop per connected region of each field mask
+  (``prepost.mask_components``) instead of one crop over all of its set pixels.
 """
 from __future__ import annotations
 
@@ -459,6 +461,18 @@ def run_unet(pil_img: Image.Image, checkpoint_path: str):
     ``None``; key order = ``FIELDS``.
     """
     from . import prepost
+    frame, mask = _segment_one(pil_img, checkpoint_path)
+    boxes = prepost.mask_bbox(mask)
+    m = mask[0].cpu().numpy()
+    masks = {f: m[i] != 0 for i, f in enumerate(FIELDS)}
+    crops = boxes_to_crops(pil_img, boxes[0].cpu().numpy(), frame)
+    return masks, crops
+
+
+def _segment_one(pil_img: Image.Image, checkpoint_path: str):
+    """The device half of ``run_unet``: ``(frame, mask)`` = the uploaded uint8 [H, W, 3 or 4] frame (``None`` for
+    other PIL modes, which are resized on the host) and the uint8 [1, 3, 512, 512] masks, both on the GPU."""
+    from . import prepost
     _require_cuda()
     _, eng = _cached_engine(checkpoint_path)
     thr = [THRESHOLDS[f] for f in FIELDS]
@@ -467,14 +481,60 @@ def run_unet(pil_img: Image.Image, checkpoint_path: str):
     if _gpu_resizable(pil_img):
         frame = _upload_rgb(pil_img)                       # uint8 [1, H, W, 3 or 4]; stays on the GPU
         x = prepost.resize_u8(frame, IMG_SIZE, IMG_SIZE, channels=3)   # the resized frame never leaves the GPU
+        frame = frame[0]
     else:
         x = torch.from_numpy(_resized_rgb_u8(pil_img.resize((IMG_SIZE, IMG_SIZE)))[None]).to(DEVICE)
     _, mask = eng.run(x, want_logits=False, thresholds=thr)
-    boxes = prepost.mask_bbox(mask)
+    return frame, mask
+
+
+def run_unet_instances(pil_img: Image.Image, checkpoint_path: str, max_instances: int = 4, min_pixels: int = 1,
+                       connectivity: int = 8):
+    """``run_unet`` with one crop per connected region of each field mask instead of one crop over all of its set
+    pixels (new, additive; ``run_unet`` itself is unchanged).  Returns ``(masks, instances)``: ``masks`` exactly as
+    ``run_unet`` returns them; ``instances[field]`` = list, largest region first, of ``{"box": (x1, y1, x2, y2),
+    "pixels": count, "crop": PIL.Image}`` for the ``max_instances`` (1..16) largest regions (``connectivity`` 4 or
+    8) of at least ``min_pixels`` pixels.  Each box is the reference's crop rectangle of the region's extent
+    (scaled to the original size, grown by 15 %, clamped); empty rectangles and near-black crops are dropped, so a
+    field may list fewer regions than it has."""
+    from . import prepost
+    frame, mask = _segment_one(pil_img, checkpoint_path)
+    comps, _ = prepost.mask_components(mask, connectivity=connectivity, max_components=max_instances)
     m = mask[0].cpu().numpy()
     masks = {f: m[i] != 0 for i, f in enumerate(FIELDS)}
-    crops = boxes_to_crops(pil_img, boxes[0].cpu().numpy(), None if frame is None else frame[0])
-    return masks, crops
+    return masks, components_to_instances(pil_img, comps[0].cpu().numpy(), frame, min_pixels)
+
+
+def components_to_instances(pil_img: Image.Image, comps: np.ndarray, frame_dev=None, min_pixels: int = 1
+                            ) -> Dict[str, List[dict]]:
+    """Component table int32 [3, K, 6] (``prepost.mask_components`` of one image's masks, rows largest first) ->
+    ``{field: [{"box", "pixels", "crop"}, ...]}``.  Rows with fewer than ``min_pixels`` pixels (or none) are left
+    out; the rest go through ``_crop_rect`` and the near-black test of :func:`boxes_to_crops` -- on the device
+    frame ``frame_dev`` when given (``prepost.box_sums``, 16 rectangles per call), else on the host."""
+    cands = []                                       # (field, rectangle, pixels, extent)
+    for i, key in enumerate(FIELDS):
+        for row in comps[i]:
+            xmin, xmax, ymin, ymax, count = (int(v) for v in row[:5])
+            if count == 0 or count < min_pixels:
+                continue
+            r = _crop_rect(pil_img.size, (xmin, xmax, ymin, ymax))
+            if r is not None:
+                cands.append((key, r, count, (xmin, xmax, ymin, ymax)))
+    out: Dict[str, List[dict]] = {key: [] for key in FIELDS}
+    if frame_dev is None:
+        for key, r, count, ext in cands:
+            crop = _crop_from_extent(pil_img, ext)
+            if crop is not None:
+                out[key].append({"box": r, "pixels": count, "crop": crop})
+        return out
+    from . import prepost
+    sums = [prepost.box_sums(frame_dev, [c[1] for c in cands[lo:lo + 16]], channels=3)
+            for lo in range(0, len(cands), 16)]
+    totals = torch.cat(sums).cpu().tolist() if sums else []
+    for (key, r, count, _), total in zip(cands, totals):
+        if total >= 3 * (r[2] - r[0]) * (r[3] - r[1]) * 3:
+            out[key].append({"box": r, "pixels": count, "crop": pil_img.crop(r)})
+    return out
 
 
 # which enhancement the app applies to which field before OCR.space (reference app_camera.py:800-811)

@@ -3,7 +3,9 @@
 * ``resize_u8``  -- ``PIL.Image.resize((512, 512))`` of reference inference.py:35,63 for uint8
   frames already on the device, bit-identical to Pillow's 8-bit bicubic resample;
 * ``mask_bbox``  -- the ``np.where(mask)`` min/max of reference inference.py:85-93 as 5 ints per
-  (image, class) instead of a 512x512 mask.
+  (image, class) instead of a 512x512 mask;
+* ``mask_components`` -- connected components of the masks (``scipy.ndimage.label`` labels, the boxes and sizes
+  of the largest regions of each plane), where ``mask_bbox`` gives one box over all set pixels.
 """
 from __future__ import annotations
 
@@ -112,6 +114,38 @@ def mask_bbox_bits(bits: torch.Tensor) -> torch.Tensor:
         nat.check(nat.lib().unetb200_mask_bbox_bits(bits.data_ptr(), n * c, h, wb * 8, out.data_ptr(),
                                                     torch.cuda.current_stream(bits.device).cuda_stream))
     return out
+
+
+def mask_components(mask: torch.Tensor, *, packed: bool = False, connectivity: int = 8, max_components: int = 8,
+                    labels: bool = False):
+    """Connected components of every plane of uint8 ``[N, C, H, W]`` masks (non-zero = set), or of bit-packed
+    ``[N, C, H, W/8]`` masks with ``packed=True`` (``Engine.run(mask_bits=True)``; ``W`` a multiple of 32).
+
+    Returns ``(comps, n)``: int32 ``[N, C, K, 6]`` = xmin, xmax, ymin, ymax, count, label of the
+    ``K = max_components`` (1..16) largest components of each plane (count descending, then label ascending;
+    unused rows W, -1, H, -1, 0, 0) and int32 ``[N, C]`` = number of components per plane.  With ``labels=True``
+    also int32 ``[N, C, H, W]``, equal to ``scipy.ndimage.label`` of each plane (4-connectivity:
+    ``generate_binary_structure(2, 1)``; 8: ``np.ones((3, 3))``).  Enqueued on the current stream."""
+    if mask.dtype != torch.uint8 or mask.dim() != 4 or not mask.is_cuda:
+        raise RuntimeError("mask_components expects a CUDA uint8 [N,C,H,W] (or [N,C,H,W/8] bit-packed) tensor")
+    mask = mask.contiguous()
+    n, c, h, wm = mask.shape
+    w = wm * 8 if packed else wm
+    lib = nat.lib()
+    ws_bytes = lib.unetb200_components_workspace_bytes(n * c, h, w)
+    if ws_bytes == 0:
+        raise RuntimeError(f"mask_components: bad mask shape {tuple(mask.shape)}")
+    dev = mask.device
+    comps = torch.empty((n, c, max(int(max_components), 1), 6), dtype=torch.int32, device=dev)
+    counts = torch.empty((n, c), dtype=torch.int32, device=dev)
+    lab = torch.empty((n, c, h, w), dtype=torch.int32, device=dev) if labels else None
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        nat.check(lib.unetb200_mask_components(
+            mask.data_ptr(), int(bool(packed)), n * c, h, w, int(connectivity), int(max_components),
+            None if lab is None else lab.data_ptr(), comps.data_ptr(), counts.data_ptr(), ws.data_ptr(), ws_bytes,
+            torch.cuda.current_stream(dev).cuda_stream))
+    return (comps, counts, lab) if labels else (comps, counts)
 
 
 def box_sums(frame: torch.Tensor, rects, channels: int = None) -> torch.Tensor:
