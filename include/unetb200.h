@@ -261,6 +261,45 @@ uint64_t unetb200_components_workspace_bytes(int n_planes, int h, int w);
 int unetb200_mask_components(const uint8_t* mask, int packed, int n_planes, int h, int w, int connectivity,
                              int max_components, int32_t* labels, int32_t* comps, int32_t* n_comps, void* workspace,
                              uint64_t workspace_bytes, void* stream);
+/* unetb200_mask_components plus the oriented box of every selected component (DESIGN.md 6b), for upright crops of
+ * tilted fields.  labels, comps and n_comps are bit-identical to unetb200_mask_components; h, w <= 32767 and
+ * n_planes <= 65535 (else UNETB200_EINVAL).
+ *   scale      nullable (= 1, 1); device float64 [n_planes][2] = (sx, sy), positive and finite: mask pixel (x, y) is
+ *              the frame point X = (x + 0.5) sx - 0.5, Y = (y + 0.5) sy - 0.5 (sx = frame width / w, ...)
+ *   moments    int64 [n_planes, max_components, 6] = n, Sx, Sy, Sxx, Sxy, Syy of the row's component's mask pixels
+ *              (cv2.moments(binaryImage=True)'s m00, m10, m01, m20, m11, m02); unused rows zeros
+ *   obox       float64 [n_planes, max_components, 6] = e1x, e1y, umin, umax, vmin, vmax: e1 = the unit principal axis
+ *              of the frame-space covariance (e1x > 0, or e1x == 0 and e1y > 0), e2 = (-e1y, e1x), and the extents of
+ *              u = X e1x + Y e1y, v = X e2x + Y e2y over the component's pixels; unused rows zeros
+ *   workspace  >= unetb200_components_oriented_workspace_bytes(n_planes, h, w) bytes (the components workspace, 16-byte
+ *              aligned, plus 512 bytes per plane), 16-byte aligned
+ * moments, obox and scale are 8-byte aligned.  Integer arithmetic and correctly rounded float64 + - * / sqrt only:
+ * the outputs are deterministic and equal oracle/oriented.py bit for bit.  The query returns 0 for a bad size. */
+uint64_t unetb200_components_oriented_workspace_bytes(int n_planes, int h, int w);
+int unetb200_mask_components_oriented(const uint8_t* mask, int packed, int n_planes, int h, int w, int connectivity,
+                                      int max_components, const double* scale, int32_t* labels, int32_t* comps,
+                                      int32_t* n_comps, int64_t* moments, double* obox, void* workspace,
+                                      uint64_t workspace_bytes, void* stream);
+/* Ragged batch of affine crops: output pixel (j, i) of crop k samples its frame at (m0 j + m1 i + m2, m3 j + m4 i + m5),
+ * bilinear with replicated borders, bit-identical to cv2.warpAffine(src, M, (out_w, out_h),
+ * flags=INTER_LINEAR | WARP_INVERSE_MAP, borderMode=BORDER_REPLICATE) of the RGB frame. */
+typedef struct unetb200_warp_crop {
+    uint64_t src;             /* device address of the frame's pixel (0, 0) */
+    int32_t src_h, src_w;     /* frame size, 1..32767 */
+    int32_t src_stride;       /* pixels per frame row, >= src_w */
+    int32_t src_pixel_bytes;  /* 3 (packed RGB) or 4 (RGBX: Pillow's storage of an RGB image); bytes 0..2 are R, G, B */
+    double m[6];              /* the inverse map M = [[m0, m1, m2], [m3, m4, m5]] (frame point of an output pixel) */
+    int32_t out_w, out_h;     /* crop size, 1..32767 */
+    uint64_t out_off;         /* byte offset of the crop's packed uint8 [out_h][out_w][3] in `out`; must not decrease
+                               * from one crop to the next, nor start inside the previous crop */
+} unetb200_warp_crop;
+/* table_host = the n descriptors (read for validation and grid sizes), table_dev = the same n structs in device
+ * memory (8-byte aligned).  out = device buffer of the crops; sums = device uint64 [n] (zeroed here), the byte sum of
+ * each crop (the near-black test of inference.py:121-125 is sum < 3 * 3 * out_w * out_h).  A bad descriptor, or a
+ * matrix that takes a coordinate of the crop to 2^19 or beyond (OpenCV's fixed point would overflow), is
+ * UNETB200_EINVAL.  Asynchronous, enqueued on `stream`; nothing is allocated. */
+int unetb200_warp_crops(const unetb200_warp_crop* table_host, const void* table_dev, int n, uint8_t* out,
+                        uint64_t* sums, void* stream);
 /* Byte sums of n_boxes (<= 16) rectangles {x1, y1, x2, y2} (half-open, host array of 4*n_boxes ints) of one
  * uint8 [h][w][c] device frame -> sums_dev uint64 [n_boxes] (zeroed here): the `np.array(crop).mean() < 3`
  * rejection of inference.py:121-125 as the exact integer test sum < 3 * (x2-x1)*(y2-y1)*c. */

@@ -51,6 +51,15 @@ class EnhCrop(C.Structure):
     ]
 
 
+class WarpCrop(C.Structure):
+    """``unetb200_warp_crop`` (include/unetb200.h): one crop of an affine-crop batch."""
+    _fields_ = [
+        ("src", C.c_uint64), ("src_h", C.c_int32), ("src_w", C.c_int32), ("src_stride", C.c_int32),
+        ("src_pixel_bytes", C.c_int32), ("m", C.c_double * 6), ("out_w", C.c_int32), ("out_h", C.c_int32),
+        ("out_off", C.c_uint64),
+    ]
+
+
 # every symbol include/unetb200.h declares: name -> (restype, argtypes)
 _VP, _I, _U64, _F = C.c_void_p, C.c_int, C.c_uint64, C.c_float
 SYMBOLS = {
@@ -92,6 +101,10 @@ SYMBOLS = {
     "unetb200_mask_bbox_bits": (_I, [_VP, _I, _I, _I, _VP, _VP]),
     "unetb200_components_workspace_bytes": (_U64, [_I, _I, _I]),
     "unetb200_mask_components": (_I, [_VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _U64, _VP]),
+    "unetb200_components_oriented_workspace_bytes": (_U64, [_I, _I, _I]),
+    "unetb200_mask_components_oriented": (_I, [_VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP,
+                                               _U64, _VP]),
+    "unetb200_warp_crops": (_I, [C.POINTER(WarpCrop), _VP, _I, _VP, _VP, _VP]),
     "unetb200_box_sums": (_I, [_VP, _I, _I, _I, C.POINTER(C.c_int32), _I, _VP, _VP]),
     "unetb200_box_sums_ps": (_I, [_VP, _I, _I, _I, _I, C.POINTER(C.c_int32), _I, _VP, _VP]),
     "unetb200_test_fastdiv": (C.c_uint32, [C.c_uint32, C.c_uint32]),

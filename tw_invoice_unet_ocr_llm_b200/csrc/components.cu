@@ -14,10 +14,15 @@
 // Every link points to a smaller raster index (parent[i] <= i), so the root of a component is its first pixel in
 // raster order and numbering the roots in raster order gives scipy.ndimage.label's labels.  All statistics are
 // integer min / max / add, so every output is independent of scheduling.
+//
+// unetb200_mask_components_oriented runs the same passes, then the oriented-box passes of the selected components
+// (cc_moments_kernel ... cc_obox_kernel, below).  Their floating-point results are min / max of values that do not
+// depend on the order of work, so they are deterministic too.
 #include "../../include/unetb200.h"
 
 #include <cuda_runtime.h>
 
+#include <climits>
 #include <cstdio>
 
 #include "errors.h"
@@ -361,39 +366,275 @@ unsigned long long work_words(int n_planes, const Plane& g) {
            (static_cast<unsigned long long>(g.n) + 5ull * g.cap + g.nseg + g.wpp);
 }
 
-}  // namespace
+// ---------------------------------------------------------------- oriented boxes of the selected components
+// (unetb200_mask_components_oriented): three more passes over the parent array after cc_select_kernel.
+//
+//   cc_moments_kernel  raw moments n, Sx, Sy, Sxx, Sxy, Syy of each selected component (int64 atomics)
+//   cc_axis_kernel     principal axis e1 of each selected row from its moments and the plane's frame scale
+//   cc_extent_kernel   min / max of the projections u = P.e1, v = P.e2 of the component's frame points P
+//   cc_obox_kernel     extents back to float64 (unused rows: zeros)
+//
+// The geometry uses integer arithmetic and correctly rounded fp64 + - * / sqrt only (__d*_rn: no FMA contraction,
+// no transcendental function), so oracle/oriented.py restates it bit for bit.
+constexpr int kMaxSide = 32767;      // h, w <= 32767: n * w^2 < 2^61, every moment sum is exact in int64
 
-extern "C" {
-
-uint64_t unetb200_components_workspace_bytes(int n_planes, int h, int w) {
-    Plane g;
-    if (n_planes <= 0 || !plane_of(h, w, &g)) return 0;
-    return 4ull * work_words(n_planes, g);
+// Workspace tail of the oriented call, behind the components workspace (16-byte aligned): [P][kMaxK][4] int64 =
+// order-preserving images of umin, umax, vmin, vmax.
+unsigned long long oriented_tail_offset(int n_planes, const Plane& g) {
+    return (4ull * work_words(n_planes, g) + 15ull) & ~15ull;
+}
+unsigned long long oriented_bytes(int n_planes, const Plane& g) {
+    return oriented_tail_offset(n_planes, g) + static_cast<unsigned long long>(n_planes) * kMaxK * 4 * 8;
 }
 
-int unetb200_mask_components(const uint8_t* mask, int packed, int n_planes, int h, int w, int connectivity,
-                             int max_components, int32_t* labels, int32_t* comps, int32_t* n_comps, void* workspace,
-                             uint64_t workspace_bytes, void* stream) {
+// Component id of pixel i (-1 = background), as cc_stats_kernel reads it after cc_number_kernel.
+__device__ __forceinline__ int pixel_id(const int* __restrict__ par, int i) {
+    const int v = par[i];
+    if (v == kBg) return -1;
+    return v < kBg ? -v - 2 : -par[v] - 2;
+}
+
+// Row of the plane's selection that holds component `id`, or -1 (ids are unique within a plane).
+__device__ __forceinline__ int slot_of(const int* sel, int k_out, int id) {
+    int s = -1;
+    if (id >= 0) {
+        for (int k = 0; k < k_out; ++k) s = sel[k] == id ? k : s;
+    }
+    return s;
+}
+
+// sel[k] = id of the plane's k-th selected component (comps[..., 5] - 1; -1 for an unused row)
+__device__ __forceinline__ void load_selection(const int32_t* __restrict__ comps, int p, int k_out, int* sel) {
+    if (threadIdx.x < kMaxK)
+        sel[threadIdx.x] = static_cast<int>(threadIdx.x) < k_out
+                               ? comps[(static_cast<size_t>(p) * k_out + threadIdx.x) * 6 + 5] - 1 : -1;
+}
+
+// Order-preserving int64 image of a double (signed compare of the images == numeric compare; -0 < +0) and back.
+__device__ __forceinline__ long long dkey(double d) {
+    const long long b = __double_as_longlong(d);
+    return b >= 0 ? b : b ^ 0x7fffffffffffffffLL;
+}
+__device__ __forceinline__ double dkey_inv(long long k) {
+    return __longlong_as_double(k >= 0 ? k : k ^ 0x7fffffffffffffffLL);
+}
+
+// One warp per row (blockIdx.y = plane, 8 rows per block), 32 columns per step.  Lanes of the same selected
+// component (__match_any_sync) add their pixels with one set of atomics from the lowest lane: the group's lanes l
+// lie in one row y at x = x0 + l, so with c = popc, S1 = sum l and S2 = sum l^2 (bit sums of the group mask)
+// Sx = c x0 + S1, Sxx = c x0^2 + 2 x0 S1 + S2, Sy = c y, Sxy = y Sx, Syy = c y^2.
+__global__ void __launch_bounds__(256) cc_moments_kernel(Plane g, const int* __restrict__ parent,
+                                                         const int32_t* __restrict__ comps, int k_out,
+                                                         unsigned long long* __restrict__ mom) {
+    __shared__ int sel[kMaxK];
+    const int p = blockIdx.y;
+    load_selection(comps, p, k_out, sel);
+    __syncthreads();
+    const int y = blockIdx.x * 8 + static_cast<int>(threadIdx.x >> 5);
+    if (y >= g.h) return;                                            // whole warps leave together
+    const int lane = threadIdx.x & 31;
+    const int* par = parent + static_cast<size_t>(p) * g.n;
+    unsigned long long* mp = mom + static_cast<size_t>(p) * k_out * 6;
+    const uint32_t bit[5] = {0xaaaaaaaau, 0xccccccccu, 0xf0f0f0f0u, 0xff00ff00u, 0xffff0000u};   // bit j of lane index
+    for (int x0 = 0; x0 < g.w; x0 += 32) {
+        const int x = x0 + lane;
+        const int slot = x < g.w ? slot_of(sel, k_out, pixel_id(par, y * g.w + x)) : -1;
+        const uint32_t grp = __match_any_sync(0xffffffffu, slot);
+        if (slot >= 0 && lane == __ffs(grp) - 1) {
+            long long s1 = 0, s2 = 0;
+#pragma unroll
+            for (int j = 0; j < 5; ++j) {
+                s1 += static_cast<long long>(__popc(grp & bit[j])) << j;
+#pragma unroll
+                for (int k = 0; k < 5; ++k) s2 += static_cast<long long>(__popc(grp & bit[j] & bit[k])) << (j + k);
+            }
+            const long long c = __popc(grp), X0 = x0, Y = y;
+            const long long sx = c * X0 + s1;
+            unsigned long long* o = mp + slot * 6;
+            atomicAdd(o + 0, static_cast<unsigned long long>(c));
+            atomicAdd(o + 1, static_cast<unsigned long long>(sx));
+            atomicAdd(o + 2, static_cast<unsigned long long>(c * Y));
+            atomicAdd(o + 3, static_cast<unsigned long long>(c * X0 * X0 + 2 * X0 * s1 + s2));
+            atomicAdd(o + 4, static_cast<unsigned long long>(sx * Y));
+            atomicAdd(o + 5, static_cast<unsigned long long>(c * Y * Y));
+        }
+    }
+}
+
+// Signed 128-bit integer -> fp64, rounded to nearest-even (as Python's float(int)): values below 2^63 go through
+// __ull2double_rn; larger ones are cut to their top 63 bits with a sticky bit for what was cut (it lies below the
+// rounding position of a 53-bit significand), converted, and scaled back by an exact power of two.
+__device__ __forceinline__ double i128_to_double_rn(__int128 v) {
+    const bool neg = v < 0;
+    const unsigned __int128 m = neg ? -static_cast<unsigned __int128>(v) : static_cast<unsigned __int128>(v);
+    double d;
+    if ((m >> 63) == 0) {
+        d = __ull2double_rn(static_cast<unsigned long long>(m));
+    } else {
+        const unsigned long long hi = static_cast<unsigned long long>(m >> 64);
+        const int s = (hi ? 128 - __clzll(static_cast<long long>(hi)) : 64) - 63;      // 1 .. 65
+        unsigned long long t = static_cast<unsigned long long>(m >> s);
+        if (m & ((static_cast<unsigned __int128>(1) << s) - 1)) t |= 1ull;
+        d = __dmul_rn(__ull2double_rn(t), __longlong_as_double(static_cast<long long>(1023 + s) << 52));
+    }
+    return neg ? -d : d;
+}
+
+// One thread per (plane, row): e1 of DESIGN 6b from the exact covariances; initialises the extent keys.
+__global__ void __launch_bounds__(256) cc_axis_kernel(int n_rows, int k_out, const double* __restrict__ scale,
+                                                      const long long* __restrict__ mom, double* __restrict__ obox,
+                                                      long long* __restrict__ keys) {
+    const int r = blockIdx.x * 256 + threadIdx.x;
+    if (r >= n_rows) return;
+    const int p = r / k_out;
+    const long long* m = mom + static_cast<size_t>(r) * 6;
+    long long* kr = keys + static_cast<size_t>(r) * 4;
+    kr[0] = LLONG_MAX; kr[1] = LLONG_MIN; kr[2] = LLONG_MAX; kr[3] = LLONG_MIN;
+    double ex = 0.0, ey = 0.0;
+    const long long n = m[0];
+    if (n > 0) {
+        const double sx = scale ? scale[2 * p] : 1.0, sy = scale ? scale[2 * p + 1] : 1.0;
+        const __int128 N = n, Sx = m[1], Sy = m[2];
+        const double cxx = i128_to_double_rn(N * m[3] - Sx * Sx);
+        const double cxy = i128_to_double_rn(N * m[4] - Sx * Sy);
+        const double cyy = i128_to_double_rn(N * m[5] - Sy * Sy);
+        const double a = __dmul_rn(__dmul_rn(sx, sx), cxx);
+        const double b = __dmul_rn(__dmul_rn(sx, sy), cxy);
+        const double c = __dmul_rn(__dmul_rn(sy, sy), cyy);
+        if (b == 0.0) {
+            ex = a >= c ? 1.0 : 0.0;
+            ey = a >= c ? 0.0 : 1.0;
+        } else {
+            const double amc = __dadd_rn(a, -c);
+            const double d = __dsqrt_rn(__dadd_rn(__dmul_rn(amc, amc), __dmul_rn(4.0, __dmul_rn(b, b))));
+            double vx, vy;
+            if (a >= c) {
+                vx = __dadd_rn(amc, d);
+                vy = __dmul_rn(2.0, b);
+            } else {
+                vx = __dmul_rn(2.0, b);
+                vy = __dadd_rn(__dadd_rn(c, -a), d);
+            }
+            const double nrm = __dsqrt_rn(__dadd_rn(__dmul_rn(vx, vx), __dmul_rn(vy, vy)));
+            ex = __ddiv_rn(vx, nrm);
+            ey = __ddiv_rn(vy, nrm);
+            if (ex < 0.0 || (ex == 0.0 && ey < 0.0)) {
+                ex = -ex;
+                ey = -ey;
+            }
+        }
+    }
+    obox[static_cast<size_t>(r) * 6 + 0] = ex;
+    obox[static_cast<size_t>(r) * 6 + 1] = ey;
+}
+
+// Frame point of a mask pixel and its projections u = X e1x + Y e1y, v = X e2x + Y e2y (e2 = (-e1y, e1x)).
+__device__ __forceinline__ void project(int x, int y, double sx, double sy, double ex, double ey, double& u,
+                                        double& v) {
+    const double X = __dadd_rn(__dmul_rn(__dadd_rn(static_cast<double>(x), 0.5), sx), -0.5);
+    const double Y = __dadd_rn(__dmul_rn(__dadd_rn(static_cast<double>(y), 0.5), sy), -0.5);
+    u = __dadd_rn(__dmul_rn(X, ex), __dmul_rn(Y, ey));
+    v = __dadd_rn(__dmul_rn(X, -ey), __dmul_rn(Y, ex));
+}
+
+// Same walk as cc_moments_kernel.  Within a row, X grows with x, Y is fixed, and a correctly rounded product with
+// a fixed factor and a correctly rounded sum with a fixed term are monotone: u and v are monotone in x along the
+// row, so a group's extremes are at its first and last lane and the lowest lane projects just those two pixels.
+__global__ void __launch_bounds__(256) cc_extent_kernel(Plane g, const int* __restrict__ parent,
+                                                        const int32_t* __restrict__ comps, int k_out,
+                                                        const double* __restrict__ scale,
+                                                        const double* __restrict__ obox, long long* __restrict__ keys) {
+    __shared__ int sel[kMaxK];
+    __shared__ double e1[kMaxK][2];
+    const int p = blockIdx.y;
+    load_selection(comps, p, k_out, sel);
+    if (threadIdx.x < static_cast<unsigned>(2 * k_out))
+        e1[threadIdx.x >> 1][threadIdx.x & 1] = obox[(static_cast<size_t>(p) * k_out + (threadIdx.x >> 1)) * 6 + (threadIdx.x & 1)];
+    __syncthreads();
+    const int y = blockIdx.x * 8 + static_cast<int>(threadIdx.x >> 5);
+    if (y >= g.h) return;
+    const int lane = threadIdx.x & 31;
+    const double sx = scale ? scale[2 * p] : 1.0, sy = scale ? scale[2 * p + 1] : 1.0;
+    const int* par = parent + static_cast<size_t>(p) * g.n;
+    long long* kp = keys + static_cast<size_t>(p) * k_out * 4;
+    for (int x0 = 0; x0 < g.w; x0 += 32) {
+        const int x = x0 + lane;
+        const int slot = x < g.w ? slot_of(sel, k_out, pixel_id(par, y * g.w + x)) : -1;
+        const uint32_t grp = __match_any_sync(0xffffffffu, slot);
+        if (slot >= 0 && lane == __ffs(grp) - 1) {
+            double u0, v0, u1, v1;
+            project(x, y, sx, sy, e1[slot][0], e1[slot][1], u0, v0);
+            project(x0 + 31 - __clz(grp), y, sx, sy, e1[slot][0], e1[slot][1], u1, v1);
+            long long* o = kp + slot * 4;
+            atomicMin(o + 0, min(dkey(u0), dkey(u1)));
+            atomicMax(o + 1, max(dkey(u0), dkey(u1)));
+            atomicMin(o + 2, min(dkey(v0), dkey(v1)));
+            atomicMax(o + 3, max(dkey(v0), dkey(v1)));
+        }
+    }
+}
+
+// One thread per (plane, row): obox[2..5] = the extents (rows without pixels: zeros).
+__global__ void __launch_bounds__(256) cc_obox_kernel(int n_rows, const long long* __restrict__ mom,
+                                                      const long long* __restrict__ keys, double* __restrict__ obox) {
+    const int r = blockIdx.x * 256 + threadIdx.x;
+    if (r >= n_rows) return;
+    const bool live = mom[static_cast<size_t>(r) * 6] > 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+        obox[static_cast<size_t>(r) * 6 + 2 + j] = live ? dkey_inv(keys[static_cast<size_t>(r) * 4 + j]) : 0.0;
+}
+
+// Outputs of the oriented call (null for unetb200_mask_components)
+struct OrientedOut {
+    const double* scale;
+    int64_t* moments;
+    double* obox;
+};
+
+// Body of both entry points: validation (every failure before any CUDA call), then the labelling passes and,
+// with `ori`, the oriented passes.  `who` prefixes the error messages.
+int components_impl(const char* who, const uint8_t* mask, int packed, int n_planes, int h, int w, int connectivity,
+                    int max_components, int32_t* labels, int32_t* comps, int32_t* n_comps, void* workspace,
+                    uint64_t workspace_bytes, void* stream, const OrientedOut* ori) {
+    char buf[240];
+    auto fail = [&](int code, const char* msg) {
+        snprintf(buf, sizeof buf, "%s: %s", who, msg);
+        return ub_fail(code, buf);
+    };
     Plane g;
     if (!mask || !comps || !n_comps || !workspace)
-        return ub_fail(UNETB200_EINVAL, "mask_components: null pointer");
+        return fail(UNETB200_EINVAL, "null pointer");
     if (connectivity != 4 && connectivity != 8)
-        return ub_fail(UNETB200_EINVAL, "mask_components: connectivity must be 4 or 8");
+        return fail(UNETB200_EINVAL, "connectivity must be 4 or 8");
     if (max_components < 1 || max_components > kMaxK)
-        return ub_fail(UNETB200_EINVAL, "mask_components: max_components must be in [1, 16]");
+        return fail(UNETB200_EINVAL, "max_components must be in [1, 16]");
     if (packed != 0 && packed != 1)
-        return ub_fail(UNETB200_EINVAL, "mask_components: packed must be 0 or 1");
+        return fail(UNETB200_EINVAL, "packed must be 0 or 1");
     if (n_planes <= 0 || !plane_of(h, w, &g))
-        return ub_fail(UNETB200_EINVAL, "mask_components: bad size (n_planes, h, w >= 1 and h * w < 2^31)");
+        return fail(UNETB200_EINVAL, "bad size (n_planes, h, w >= 1 and h * w < 2^31)");
     if (packed && (w & 31))
-        return ub_fail(UNETB200_EINVAL, "mask_components: bit-packed planes need w % 32 == 0");
+        return fail(UNETB200_EINVAL, "bit-packed planes need w % 32 == 0");
     if (((packed ? reinterpret_cast<uintptr_t>(mask) : 0) | reinterpret_cast<uintptr_t>(labels) |
          reinterpret_cast<uintptr_t>(comps) | reinterpret_cast<uintptr_t>(n_comps)) & 3 ||
         (reinterpret_cast<uintptr_t>(workspace) & 15))
-        return ub_fail(UNETB200_EINVAL, "mask_components: misaligned pointer (int32 outputs and bit-packed planes "
-                                        "4-byte aligned, workspace 16-byte aligned)");
-    if (workspace_bytes < 4ull * work_words(n_planes, g))
-        return ub_fail(UNETB200_ENOMEM, "mask_components: workspace smaller than unetb200_components_workspace_bytes");
+        return fail(UNETB200_EINVAL, "misaligned pointer (int32 outputs and bit-packed planes "
+                                     "4-byte aligned, workspace 16-byte aligned)");
+    if (ori) {
+        if (!ori->moments || !ori->obox)
+            return fail(UNETB200_EINVAL, "null pointer");
+        if ((reinterpret_cast<uintptr_t>(ori->moments) | reinterpret_cast<uintptr_t>(ori->obox) |
+             reinterpret_cast<uintptr_t>(ori->scale)) & 7)
+            return fail(UNETB200_EINVAL, "misaligned pointer (moments, obox and scale 8-byte aligned)");
+        if (h > kMaxSide || w > kMaxSide)
+            return fail(UNETB200_EINVAL, "planes larger than 32767 pixels on a side");
+        if (n_planes > 65535)
+            return fail(UNETB200_EINVAL, "batch too large (at most 65535 planes)");
+        if (workspace_bytes < oriented_bytes(n_planes, g))
+            return fail(UNETB200_ENOMEM, "workspace smaller than unetb200_components_oriented_workspace_bytes");
+    } else if (workspace_bytes < 4ull * work_words(n_planes, g)) {
+        return fail(UNETB200_ENOMEM, "workspace smaller than unetb200_components_workspace_bytes");
+    }
     const int tiles_x = (w + kTileW - 1) / kTileW, tiles_y = (h + kTileH - 1) / kTileH;
     const long long tiles = static_cast<long long>(tiles_x) * tiles_y;
     const long long n_rows = static_cast<long long>(n_planes) * h;
@@ -401,7 +642,7 @@ int unetb200_mask_components(const uint8_t* mask, int packed, int n_planes, int 
     const long long pack_blocks = (static_cast<long long>(n_planes) * g.wpp * 32 + 255) / 256;
     if (tiles * n_planes >= (1LL << 31) || n_rows >= (1LL << 31) || seg_blocks >= (1LL << 31) ||
         pack_blocks >= (1LL << 31))
-        return ub_fail(UNETB200_EINVAL, "mask_components: batch too large");
+        return fail(UNETB200_EINVAL, "batch too large");
 
     int* base = static_cast<int*>(workspace);
     const size_t pn = static_cast<size_t>(n_planes) * g.n, pc = static_cast<size_t>(n_planes) * g.cap;
@@ -439,13 +680,61 @@ int unetb200_mask_components(const uint8_t* mask, int packed, int n_planes, int 
     cc_stats_kernel<<<static_cast<unsigned>((n_rows + 7) / 8), 256, 0, s>>>(g, static_cast<int>(n_rows), wk.parent,
                                                                             wk, labels);
     cc_select_kernel<<<static_cast<unsigned>(n_planes), 256, 0, s>>>(g, wk, n_comps, max_components, comps);
+    if (ori) {
+        const int k = max_components, rows = n_planes * k;
+        long long* keys = reinterpret_cast<long long*>(static_cast<char*>(workspace) + oriented_tail_offset(n_planes, g));
+        const dim3 walk(static_cast<unsigned>((h + 7) / 8), static_cast<unsigned>(n_planes));
+        const unsigned row_blocks = static_cast<unsigned>((rows + 255) / 256);
+        cudaError_t e = cudaMemsetAsync(ori->moments, 0, static_cast<size_t>(rows) * 6 * sizeof(int64_t), s);
+        if (e != cudaSuccess) {
+            snprintf(buf, sizeof buf, "%s: memset failed: %s", who, cudaGetErrorString(e));
+            return ub_fail(UNETB200_ECUDA, buf);
+        }
+        auto* mom = reinterpret_cast<unsigned long long*>(ori->moments);
+        const auto* smom = reinterpret_cast<const long long*>(ori->moments);
+        cc_moments_kernel<<<walk, 256, 0, s>>>(g, wk.parent, comps, k, mom);
+        cc_axis_kernel<<<row_blocks, 256, 0, s>>>(rows, k, ori->scale, smom, ori->obox, keys);
+        cc_extent_kernel<<<walk, 256, 0, s>>>(g, wk.parent, comps, k, ori->scale, ori->obox, keys);
+        cc_obox_kernel<<<row_blocks, 256, 0, s>>>(rows, smom, keys, ori->obox);
+    }
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {
-        char buf[200];
-        snprintf(buf, sizeof buf, "mask_components: launch failed: %s", cudaGetErrorString(e));
+        snprintf(buf, sizeof buf, "%s: launch failed: %s", who, cudaGetErrorString(e));
         return ub_fail(UNETB200_ECUDA, buf);
     }
     return UNETB200_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+uint64_t unetb200_components_workspace_bytes(int n_planes, int h, int w) {
+    Plane g;
+    if (n_planes <= 0 || !plane_of(h, w, &g)) return 0;
+    return 4ull * work_words(n_planes, g);
+}
+
+uint64_t unetb200_components_oriented_workspace_bytes(int n_planes, int h, int w) {
+    Plane g;
+    if (n_planes <= 0 || n_planes > 65535 || h > kMaxSide || w > kMaxSide || !plane_of(h, w, &g)) return 0;
+    return oriented_bytes(n_planes, g);
+}
+
+int unetb200_mask_components(const uint8_t* mask, int packed, int n_planes, int h, int w, int connectivity,
+                             int max_components, int32_t* labels, int32_t* comps, int32_t* n_comps, void* workspace,
+                             uint64_t workspace_bytes, void* stream) {
+    return components_impl("mask_components", mask, packed, n_planes, h, w, connectivity, max_components, labels,
+                           comps, n_comps, workspace, workspace_bytes, stream, nullptr);
+}
+
+int unetb200_mask_components_oriented(const uint8_t* mask, int packed, int n_planes, int h, int w, int connectivity,
+                                      int max_components, const double* scale, int32_t* labels, int32_t* comps,
+                                      int32_t* n_comps, int64_t* moments, double* obox, void* workspace,
+                                      uint64_t workspace_bytes, void* stream) {
+    const OrientedOut ori{scale, moments, obox};
+    return components_impl("mask_components_oriented", mask, packed, n_planes, h, w, connectivity, max_components,
+                           labels, comps, n_comps, workspace, workspace_bytes, stream, &ori);
 }
 
 }  // extern "C"

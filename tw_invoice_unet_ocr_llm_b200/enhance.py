@@ -146,6 +146,33 @@ def enhance_windows(frame: torch.Tensor, rects: Sequence[tuple], kinds: Sequence
         return _execute(table, n, d_tab.data_ptr(), frame.data_ptr(), ob.value, wb.value, dev, (d_tab, frame))
 
 
+def enhance_packed(buf: torch.Tensor, offsets: Sequence[int], sizes: Sequence[tuple], kinds: Sequence
+                   ) -> List[np.ndarray]:
+    """Enhance packed uint8 ``[h][w][3]`` RGB crops that are already in the device buffer ``buf`` (1-D uint8) at byte
+    ``offsets`` -- the upright crops of ``prepost.warp_crops`` -- in place: only the descriptors go up.  ``sizes``:
+    ``(w, h)`` per crop.  Same results as :func:`enhance_batch` of the same crops."""
+    if buf.dtype != torch.uint8 or buf.dim() != 1 or not buf.is_cuda or not buf.is_contiguous():
+        raise RuntimeError("enhance_packed expects a contiguous CUDA uint8 1-D buffer")
+    if not (len(offsets) == len(sizes) == len(kinds)):
+        raise ValueError("offsets, sizes and kinds differ in length")
+    if not offsets:
+        return []
+    n = len(offsets)
+    table = (nat.EnhCrop * n)()
+    for t, off, (w, h), kind in zip(table, offsets, sizes, kinds):
+        off, w, h = int(off), int(w), int(h)
+        if off < 0 or w <= 0 or h <= 0 or off + 3 * w * h > buf.numel():
+            raise ValueError(f"crop of {w}x{h} at byte {off} outside the {buf.numel()}-byte buffer")
+        t.flags, t.clip = _recipe(kind)
+        t.h, t.w, t.src_stride, t.src_pixel_bytes, t.src_off = h, w, w, 3, off
+    sb, ob, wb = C.c_uint64(), C.c_uint64(), C.c_uint64()
+    nat.check(nat.lib().unetb200_enhance_plan(table, n, C.byref(sb), C.byref(ob), C.byref(wb)))
+    dev = buf.device
+    with torch.cuda.device(dev):
+        d_tab = torch.frombuffer(bytearray(table), dtype=torch.uint8).to(dev)
+        return _execute(table, n, d_tab.data_ptr(), buf.data_ptr(), ob.value, wb.value, dev, (d_tab, buf))
+
+
 def enhance_for_ocrspace(pil_crop, mode: str = "text"):
     """Reference app_camera.py:572-598: ``mode="text"`` binarises (invoice number, date), any other
     mode returns the contrast-enhanced gray image (total amount)."""

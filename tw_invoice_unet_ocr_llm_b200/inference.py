@@ -17,10 +17,13 @@ keeps working unmodified.  Differences, all internal:
 * ``run_unet_batch`` (new, additive) does the same for a list of images in one
   batched forward.
 * ``run_unet_instances`` (new, additive) returns one crop per connected region of each field mask
-  (``prepost.mask_components``) instead of one crop over all of its set pixels.
+  (``prepost.mask_components``) instead of one crop over all of its set pixels; with ``deskew=True`` each crop
+  is cut upright along the region's principal axis (``prepost.mask_components_oriented`` +
+  ``prepost.warp_crops``), and ``enhance=True`` adds the OCR enhancement of each crop.
 """
 from __future__ import annotations
 
+import math
 import os
 import threading
 from typing import Dict, List, Optional, Sequence, Tuple
@@ -131,6 +134,40 @@ def _crop_rect(size, extent):
     if x2 <= x1 or y2 <= y1:
         return None
     return x1, y1, x2, y2
+
+
+def _oriented_crop(obox, scale) -> dict:
+    """Oriented box of a region (``obox`` = e1x, e1y, umin, umax, vmin, vmax from
+    ``prepost.mask_components_oriented``; ``scale`` = (sx, sy) frame pixels per mask pixel) -> its upright crop
+    (DESIGN.md 6b):
+
+    * ``"size"`` ``(L, Wd)``: the extents along e1 and e2 = (-e1y, e1x), widened by one mask pixel block
+      (half sizes ``hu = (|e1x| sx + |e1y| sy) / 2``, ``hv = (|e2x| sx + |e2y| sy) / 2`` on each side);
+    * ``"out_size"`` ``(out_w, out_h) = (max(1, ceil(1.3 L)), max(1, ceil(1.3 Wd)))``: the reference's 15 % growth on
+      each side, one output pixel per frame pixel;
+    * ``"M"``: the inverse 2x3 map, output pixel (j, i) samples frame point ``o + j e1 + i e2``, where ``o`` puts the
+      box centre ``c = (umin + umax) / 2 e1 + (vmin + vmax) / 2 e2`` in the middle of the crop;
+    * ``"quad"``: the crop's four outer corners in the frame (top-left, top-right, bottom-right, bottom-left of the
+      crop), ``"angle"``: ``degrees(atan2(e1y, e1x))`` in (-90, 90], for reporting.
+
+    A 180 degree turn cannot be told from the masks: upside-down text stays upside down."""
+    e1x, e1y, umin, umax, vmin, vmax = (float(v) for v in obox)
+    sx, sy = float(scale[0]), float(scale[1])
+    e2x, e2y = -e1y, e1x
+    hu = 0.5 * (abs(e1x) * sx + abs(e1y) * sy)
+    hv = 0.5 * (abs(e2x) * sx + abs(e2y) * sy)
+    length = umax - umin + 2.0 * hu
+    width = vmax - vmin + 2.0 * hv
+    out_w = max(1, math.ceil(1.3 * length))
+    out_h = max(1, math.ceil(1.3 * width))
+    cu, cv = 0.5 * (umin + umax), 0.5 * (vmin + vmax)
+    cx, cy = cu * e1x + cv * e2x, cu * e1y + cv * e2y
+    ox = cx - 0.5 * (out_w - 1) * e1x - 0.5 * (out_h - 1) * e2x
+    oy = cy - 0.5 * (out_w - 1) * e1y - 0.5 * (out_h - 1) * e2y
+    quad = tuple((ox + j * e1x + i * e2x, oy + j * e1y + i * e2y)
+                 for j, i in ((-0.5, -0.5), (out_w - 0.5, -0.5), (out_w - 0.5, out_h - 0.5), (-0.5, out_h - 0.5)))
+    return {"M": np.array([[e1x, e2x, ox], [e1y, e2y, oy]], np.float64), "out_size": (out_w, out_h),
+            "size": (length, width), "quad": quad, "angle": math.degrees(math.atan2(e1y, e1x))}
 
 
 def _crop_from_extent(pil_img: Image.Image, extent) -> Optional[Image.Image]:
@@ -489,20 +526,98 @@ def _segment_one(pil_img: Image.Image, checkpoint_path: str):
 
 
 def run_unet_instances(pil_img: Image.Image, checkpoint_path: str, max_instances: int = 4, min_pixels: int = 1,
-                       connectivity: int = 8):
+                       connectivity: int = 8, deskew: bool = False, enhance: bool = False):
     """``run_unet`` with one crop per connected region of each field mask instead of one crop over all of its set
     pixels (new, additive; ``run_unet`` itself is unchanged).  Returns ``(masks, instances)``: ``masks`` exactly as
     ``run_unet`` returns them; ``instances[field]`` = list, largest region first, of ``{"box": (x1, y1, x2, y2),
     "pixels": count, "crop": PIL.Image}`` for the ``max_instances`` (1..16) largest regions (``connectivity`` 4 or
     8) of at least ``min_pixels`` pixels.  Each box is the reference's crop rectangle of the region's extent
     (scaled to the original size, grown by 15 %, clamped); empty rectangles and near-black crops are dropped, so a
-    field may list fewer regions than it has."""
+    field may list fewer regions than it has.
+
+    ``deskew=True``: each ``"crop"`` is instead the upright RGB crop of the region along its principal axis
+    (:func:`_oriented_crop`), sampled on the GPU from the uploaded frame (``prepost.warp_crops``, equal to
+    ``cv2.warpAffine`` with bilinear sampling; the frame's edge pixels repeat where the crop reaches past it), and
+    each instance gains ``"quad"`` (the crop's four corners in the frame), ``"angle"`` (degrees, in (-90, 90]) and
+    ``"size"`` (the region's length and width in frame pixels).  The near-black test applies to the upright crop.
+    ``enhance=True`` adds ``"enhanced"``: the mode-"L" OCR enhancement (four times the crop size) of the crop, with
+    the field's ``ENHANCE_KINDS`` recipe, computed on the device from the crop's pixels there."""
     from . import prepost
     frame, mask = _segment_one(pil_img, checkpoint_path)
-    comps, _ = prepost.mask_components(mask, connectivity=connectivity, max_components=max_instances)
-    m = mask[0].cpu().numpy()
-    masks = {f: m[i] != 0 for i, f in enumerate(FIELDS)}
-    return masks, components_to_instances(pil_img, comps[0].cpu().numpy(), frame, min_pixels)
+    m_cpu = None
+    if not deskew:
+        comps, _ = prepost.mask_components(mask, connectivity=connectivity, max_components=max_instances)
+        m_cpu = mask[0].cpu().numpy()
+        inst = components_to_instances(pil_img, comps[0].cpu().numpy(), frame, min_pixels)
+        if enhance:
+            _enhance_instances(inst, frame)
+    else:
+        scale = (pil_img.size[0] / IMG_SIZE, pil_img.size[1] / IMG_SIZE)
+        comps, _, _, obox = prepost.mask_components_oriented(mask, connectivity=connectivity,
+                                                             max_components=max_instances, scale=scale)
+        m_cpu = mask[0].cpu().numpy()
+        if frame is None:                              # other PIL modes: the RGB conversion goes up for the warp
+            frame = _upload_rgb(pil_img.convert("RGB"))[0]
+        inst = _deskewed_instances(pil_img, comps[0].cpu().numpy(), obox[0].cpu().numpy(), frame, scale,
+                                   min_pixels, enhance)
+    masks = {f: m_cpu[i] != 0 for i, f in enumerate(FIELDS)}
+    return masks, inst
+
+
+def _deskewed_instances(pil_img: Image.Image, comps: np.ndarray, obox: np.ndarray, frame_dev: torch.Tensor, scale,
+                        min_pixels: int, enhance: bool) -> Dict[str, List[dict]]:
+    """Rows of ``prepost.mask_components_oriented`` for one image -> instances with upright crops: the rows
+    :func:`components_to_instances` would keep, each warped from the device frame in one batch; near-black upright
+    crops are dropped on their device sums; with ``enhance`` the enhancement reads the warped buffer in place."""
+    from . import prepost
+    cands = []                                       # (field, rectangle, pixels, oriented crop)
+    for i, key in enumerate(FIELDS):
+        for row, ob in zip(comps[i], obox[i]):
+            xmin, xmax, ymin, ymax, count = (int(v) for v in row[:5])
+            if count == 0 or count < min_pixels:
+                continue
+            r = _crop_rect(pil_img.size, (xmin, xmax, ymin, ymax))
+            if r is not None:
+                cands.append((key, r, count, _oriented_crop(ob, scale)))
+    out: Dict[str, List[dict]] = {key: [] for key in FIELDS}
+    if not cands:
+        return out
+    buf, offs, sizes, sums = prepost._warp_batch(frame_dev, [c[3]["M"] for c in cands],
+                                                 [c[3]["out_size"] for c in cands])
+    keep = [k for k, t in enumerate(sums.cpu().tolist()) if t >= 3 * 3 * sizes[k][0] * sizes[k][1]]
+    if not keep:
+        return out
+    host = buf.cpu().numpy()
+    enh = None
+    if enhance:
+        from . import enhance as enh_mod
+        enh = enh_mod.enhance_packed(buf, [offs[k] for k in keep], [sizes[k] for k in keep],
+                                     [ENHANCE_KINDS[cands[k][0]] for k in keep])
+    for n_kept, k in enumerate(keep):
+        key, r, count, oc = cands[k]
+        w, h = sizes[k]
+        d = {"box": r, "pixels": count, "crop": Image.fromarray(host[offs[k]:offs[k] + 3 * w * h].reshape(h, w, 3)),
+             "quad": oc["quad"], "angle": oc["angle"], "size": oc["size"]}
+        if enh is not None:
+            d["enhanced"] = Image.fromarray(enh[n_kept])
+        out[key].append(d)
+    return out
+
+
+def _enhance_instances(inst: Dict[str, List[dict]], frame_dev=None) -> None:
+    """Adds ``"enhanced"`` to every instance of :func:`components_to_instances`: the enhancement kernels read the
+    boxes straight from the device frame when there is one (as ``run_unet_enhanced`` does), else the host crops."""
+    from . import enhance
+    items = [(key, d) for key, lst in inst.items() for d in lst]
+    if not items:
+        return
+    kinds = [ENHANCE_KINDS[key] for key, _ in items]
+    if frame_dev is not None:
+        arrs = enhance.enhance_windows(frame_dev, [d["box"] for _, d in items], kinds)
+    else:
+        arrs = enhance.enhance_batch([d["crop"] for _, d in items], kinds)
+    for (_, d), a in zip(items, arrs):
+        d["enhanced"] = Image.fromarray(a)
 
 
 def components_to_instances(pil_img: Image.Image, comps: np.ndarray, frame_dev=None, min_pixels: int = 1

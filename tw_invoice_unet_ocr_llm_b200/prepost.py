@@ -5,7 +5,11 @@
 * ``mask_bbox``  -- the ``np.where(mask)`` min/max of reference inference.py:85-93 as 5 ints per
   (image, class) instead of a 512x512 mask;
 * ``mask_components`` -- connected components of the masks (``scipy.ndimage.label`` labels, the boxes and sizes
-  of the largest regions of each plane), where ``mask_bbox`` gives one box over all set pixels.
+  of the largest regions of each plane), where ``mask_bbox`` gives one box over all set pixels;
+* ``mask_components_oriented`` -- the same plus the moments and the oriented box (principal axis and extents in
+  frame coordinates) of every listed region;
+* ``warp_crops`` -- a ragged batch of affine crops of device frames, bit-identical to ``cv2.warpAffine``
+  (``INTER_LINEAR | WARP_INVERSE_MAP``, ``BORDER_REPLICATE``), with the byte sum of each crop.
 """
 from __future__ import annotations
 
@@ -146,6 +150,115 @@ def mask_components(mask: torch.Tensor, *, packed: bool = False, connectivity: i
             None if lab is None else lab.data_ptr(), comps.data_ptr(), counts.data_ptr(), ws.data_ptr(), ws_bytes,
             torch.cuda.current_stream(dev).cuda_stream))
     return (comps, counts, lab) if labels else (comps, counts)
+
+
+def _plane_scale(scale, n: int, c: int, dev) -> torch.Tensor:
+    """``scale`` of :func:`mask_components_oriented` -> float64 ``[n, c, 2]`` on ``dev`` (``None`` stays ``None``)."""
+    if scale is None:
+        return None
+    arr = np.asarray(scale.detach().cpu() if torch.is_tensor(scale) else scale, dtype=np.float64)
+    if arr.shape == (2,):
+        arr = np.broadcast_to(arr, (n, c, 2))
+    elif arr.shape == (n, 2):
+        arr = np.broadcast_to(arr[:, None], (n, c, 2))
+    elif arr.shape != (n, c, 2):
+        raise ValueError(f"scale must be (sx, sy), [N, 2] or [N, C, 2]; got shape {arr.shape}")
+    if not (np.isfinite(arr).all() and (arr > 0).all()):
+        raise ValueError("scale factors must be positive and finite")
+    return torch.from_numpy(np.ascontiguousarray(arr)).to(dev)
+
+
+def mask_components_oriented(mask: torch.Tensor, *, packed: bool = False, connectivity: int = 8,
+                             max_components: int = 8, scale=None, labels: bool = False):
+    """:func:`mask_components` plus the oriented box of each listed component (DESIGN.md 6b).
+
+    ``scale``: ``(sx, sy)`` for every plane, or per image ``[N, 2]`` / per plane ``[N, C, 2]`` (default 1, 1): the
+    size of a mask pixel in frame pixels, ``(frame_w / W, frame_h / H)`` for masks of a resized frame.  Mask pixel
+    ``(x, y)`` stands for the frame point ``((x + 0.5) sx - 0.5, (y + 0.5) sy - 0.5)``.
+
+    Returns ``(comps, n, moments, obox)`` (and the labels last with ``labels=True``): ``comps`` and ``n`` exactly as
+    :func:`mask_components`; int64 ``[N, C, K, 6]`` = n, Sx, Sy, Sxx, Sxy, Syy, the raw moments of each row's mask
+    pixels; float64 ``[N, C, K, 6]`` = e1x, e1y, umin, umax, vmin, vmax: the unit principal axis ``e1`` of the
+    frame-space covariance (``e1x > 0``, or ``e1x == 0`` and ``e1y > 0``) and the extents of the frame points
+    projected on ``e1`` and ``e2 = (-e1y, e1x)``.  Unused rows are zeros.  Planes up to 32767 pixels on a side.
+    Enqueued on the current stream."""
+    if mask.dtype != torch.uint8 or mask.dim() != 4 or not mask.is_cuda:
+        raise RuntimeError("mask_components_oriented expects a CUDA uint8 [N,C,H,W] (or [N,C,H,W/8] bit-packed) "
+                           "tensor")
+    mask = mask.contiguous()
+    n, c, h, wm = mask.shape
+    w = wm * 8 if packed else wm
+    lib = nat.lib()
+    ws_bytes = lib.unetb200_components_oriented_workspace_bytes(n * c, h, w)
+    if ws_bytes == 0:
+        raise RuntimeError(f"mask_components_oriented: bad mask shape {tuple(mask.shape)}")
+    dev = mask.device
+    sc = _plane_scale(scale, n, c, dev)
+    k = max(int(max_components), 1)
+    comps = torch.empty((n, c, k, 6), dtype=torch.int32, device=dev)
+    counts = torch.empty((n, c), dtype=torch.int32, device=dev)
+    mom = torch.empty((n, c, k, 6), dtype=torch.int64, device=dev)
+    obox = torch.empty((n, c, k, 6), dtype=torch.float64, device=dev)
+    lab = torch.empty((n, c, h, w), dtype=torch.int32, device=dev) if labels else None
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        nat.check(lib.unetb200_mask_components_oriented(
+            mask.data_ptr(), int(bool(packed)), n * c, h, w, int(connectivity), int(max_components),
+            None if sc is None else sc.data_ptr(), None if lab is None else lab.data_ptr(), comps.data_ptr(),
+            counts.data_ptr(), mom.data_ptr(), obox.data_ptr(), ws.data_ptr(), ws_bytes,
+            torch.cuda.current_stream(dev).cuda_stream))
+    return (comps, counts, mom, obox, lab) if labels else (comps, counts, mom, obox)
+
+
+def _warp_batch(frames, mats, sizes):
+    """Validated batch of :func:`warp_crops` -> (buffer uint8 [total], byte offsets, (out_w, out_h) sizes, sums)."""
+    n = len(sizes)
+    if isinstance(frames, torch.Tensor):
+        frames = [frames] * n
+    frames = list(frames)
+    mats = np.asarray(mats, dtype=np.float64)
+    if len(frames) != n or mats.shape != (n, 2, 3):
+        raise ValueError(f"warp_crops: {len(frames)} frames, matrices of shape {mats.shape} and {n} sizes do not "
+                         "describe the same crops (one frame, one 2x3 matrix and one (w, h) per crop)")
+    if n == 0:
+        raise ValueError("warp_crops: no crops")
+    dev = frames[0].device
+    for f in frames:
+        if (f.dtype != torch.uint8 or f.dim() != 3 or f.shape[2] not in (3, 4) or not f.is_cuda
+                or not f.is_contiguous() or f.device != dev):
+            raise RuntimeError("warp_crops expects contiguous CUDA uint8 [H,W,3] or [H,W,4] frames on one device")
+    table = (nat.WarpCrop * n)()
+    offs, total = [], 0
+    for t, f, m, (ow, oh) in zip(table, frames, mats, sizes):
+        ow, oh = int(ow), int(oh)
+        t.src, t.src_h, t.src_w = f.data_ptr(), int(f.shape[0]), int(f.shape[1])
+        t.src_stride, t.src_pixel_bytes = int(f.shape[1]), int(f.shape[2])
+        t.m[:] = [float(v) for v in m.reshape(-1)]
+        t.out_w, t.out_h, t.out_off = ow, oh, total
+        offs.append(total)
+        total += 3 * max(ow, 0) * max(oh, 0)
+    buf = torch.empty((max(total, 1),), dtype=torch.uint8, device=dev)
+    sums = torch.empty((n,), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        d_tab = torch.frombuffer(bytearray(table), dtype=torch.uint8).to(dev)
+        nat.check(nat.lib().unetb200_warp_crops(table, d_tab.data_ptr(), n, buf.data_ptr(), sums.data_ptr(),
+                                                torch.cuda.current_stream(dev).cuda_stream))
+    return buf, offs, [(int(w), int(h)) for w, h in sizes], sums
+
+
+def warp_crops(frames, mats, sizes):
+    """Ragged batch of upright (or any affine) crops of frames already on the device.
+
+    ``frames``: one contiguous CUDA uint8 ``[H, W, 3]`` (RGB) or ``[H, W, 4]`` (RGBX) frame for all crops, or a
+    sequence with one per crop; ``mats``: per crop the inverse 2x3 map ``M`` (output pixel ``(j, i)`` samples the
+    frame at ``M @ (j, i, 1)``); ``sizes``: per crop ``(out_w, out_h)``.  Each crop equals
+    ``cv2.warpAffine(frame_rgb, M, (out_w, out_h), flags=cv2.INTER_LINEAR | cv2.WARP_INVERSE_MAP,
+    borderMode=cv2.BORDER_REPLICATE)`` bit for bit.
+
+    Returns ``(crops, sums)``: uint8 ``[out_h, out_w, 3]`` views into one device buffer, and int64 ``[n]`` byte sums
+    on the device (a crop is near-black when ``sum < 3 * 3 * out_w * out_h``).  Enqueued on the current stream."""
+    buf, offs, sz, sums = _warp_batch(frames, mats, sizes)
+    return [buf[o:o + 3 * w * h].view(h, w, 3) for o, (w, h) in zip(offs, sz)], sums
 
 
 def box_sums(frame: torch.Tensor, rects, channels: int = None) -> torch.Tensor:
