@@ -280,6 +280,32 @@ int unetb200_mask_components_oriented(const uint8_t* mask, int packed, int n_pla
                                       int max_components, const double* scale, int32_t* labels, int32_t* comps,
                                       int32_t* n_comps, int64_t* moments, double* obox, void* workspace,
                                       uint64_t workspace_bytes, void* stream);
+/* Binary morphology of mask planes, for cleaning the field masks before unetb200_mask_components: */
+enum {
+    UNETB200_MORPH_ERODE = 0,      /* cv2.erode(m, ones((kh, kw))): AND over the window */
+    UNETB200_MORPH_DILATE = 1,     /* cv2.dilate(m, ones((kh, kw))): OR over the window */
+    UNETB200_MORPH_OPEN = 2,       /* cv2.morphologyEx(MORPH_OPEN) = dilate(erode(m)) */
+    UNETB200_MORPH_CLOSE = 3,      /* cv2.morphologyEx(MORPH_CLOSE) = erode(dilate(m)) */
+    UNETB200_MORPH_FILL_HOLES = 4  /* scipy.ndimage.binary_fill_holes(m): kw, kh ignored */
+};
+/* Workspace of unetb200_mask_morph: two bit planes for ERODE .. CLOSE (ceil(w / 32) * 4 bytes per row each), the
+ * components workspace (unetb200_components_workspace_bytes) for FILL_HOLES; 0 for a bad size or op. */
+uint64_t unetb200_morph_workspace_bytes(int n_planes, int h, int w, int op);
+/* in -> out for every plane, bit-exact with OpenCV's defaults (and SciPy's for FILL_HOLES):
+ *   element    kw x kh rectangle, 1 <= kw, kh <= 63, anchor (kw / 2, kh / 2); erosion and dilation both use the
+ *              window x - kw/2 .. x + kw - 1 - kw/2, y - kh/2 .. y + kh - 1 - kh/2 (OpenCV does not reflect the
+ *              element for dilation; SciPy does, so the two differ for even sizes)
+ *   border     pixels outside the plane take no part (BORDER_CONSTANT with morphologyDefaultBorderValue)
+ *   holes      4-connected background components that touch no border pixel become set
+ *   in, out    byte planes uint8 [n_planes, h, w] (non-zero = set; out is 0 / 1) or, with in_packed / out_packed = 1,
+ *              bit-packed planes uint8 [n_planes, h, w/8] in the format of unetb200_forward_bits (w % 32 == 0,
+ *              4-byte aligned); any of the four combinations.  In place (in == out, or any overlap) works.
+ *   workspace  >= unetb200_morph_workspace_bytes(n_planes, h, w, op) bytes, 16-byte aligned, no initialisation
+ * h, w >= 1 and h * w < 2^31 as unetb200_mask_components.  Deterministic bits.  Asynchronous: enqueued on `stream`,
+ * nothing is allocated.  A null pointer, a bad op, k, size or packed flag, or a misaligned pointer is UNETB200_EINVAL;
+ * a short workspace UNETB200_ENOMEM. */
+int unetb200_mask_morph(const uint8_t* in, int in_packed, uint8_t* out, int out_packed, int n_planes, int h, int w,
+                        int op, int kw, int kh, void* workspace, uint64_t workspace_bytes, void* stream);
 /* Ragged batch of affine crops: output pixel (j, i) of crop k samples its frame at (m0 j + m1 i + m2, m3 j + m4 i + m5),
  * bilinear with replicated borders, bit-identical to cv2.warpAffine(src, M, (out_w, out_h),
  * flags=INTER_LINEAR | WARP_INVERSE_MAP, borderMode=BORDER_REPLICATE) of the RGB frame. */

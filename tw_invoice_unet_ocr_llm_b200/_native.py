@@ -19,6 +19,7 @@ STEM, CONV3X3, CONVT2X2, HEAD = 0, 1, 2, 3
 X_F32_NCHW, X_U8_NHWC, X_F16_NCHW, X_BF16_NCHW, X_F32_NHWC, X_F16_NHWC, X_BF16_NHWC = range(7)
 LOGITS_F32, LOGITS_F16, LOGITS_BF16 = 0, 1, 2
 A_TAP, A_COL3, A_HALO = 0, 1, 2
+MORPH_ERODE, MORPH_DILATE, MORPH_OPEN, MORPH_CLOSE, MORPH_FILL_HOLES = range(5)
 
 
 class Arch(C.Structure):
@@ -104,6 +105,8 @@ SYMBOLS = {
     "unetb200_components_oriented_workspace_bytes": (_U64, [_I, _I, _I]),
     "unetb200_mask_components_oriented": (_I, [_VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP,
                                                _U64, _VP]),
+    "unetb200_morph_workspace_bytes": (_U64, [_I, _I, _I, _I]),
+    "unetb200_mask_morph": (_I, [_VP, _I, _VP, _I, _I, _I, _I, _I, _I, _I, _VP, _U64, _VP]),
     "unetb200_warp_crops": (_I, [C.POINTER(WarpCrop), _VP, _I, _VP, _VP, _VP]),
     "unetb200_box_sums": (_I, [_VP, _I, _I, _I, C.POINTER(C.c_int32), _I, _VP, _VP]),
     "unetb200_box_sums_ps": (_I, [_VP, _I, _I, _I, _I, C.POINTER(C.c_int32), _I, _VP, _VP]),

@@ -18,6 +18,11 @@
 // unetb200_mask_components_oriented runs the same passes, then the oriented-box passes of the selected components
 // (cc_moments_kernel ... cc_obox_kernel, below).  Their floating-point results are min / max of values that do not
 // depend on the order of work, so they are deterministic too.
+//
+// cc_fill_holes (unetb200_mask_morph, op UNETB200_MORPH_FILL_HOLES) labels the complement of the planes with the
+// same union-find: cc_pack_kernel in a complement mode, cc_local / cc_merge (4-connectivity) and cc_flatten, then
+// cc_border_kernel marks the roots of the components that reach the border and cc_fill_kernel writes the planes
+// with every unmarked background component set.
 #include "../../include/unetb200.h"
 
 #include <cuda_runtime.h>
@@ -25,6 +30,7 @@
 #include <climits>
 #include <cstdio>
 
+#include "cc_internal.h"
 #include "errors.h"
 
 namespace {
@@ -34,6 +40,11 @@ constexpr int kSeg = 1024;                     // raster pixels per root-count s
 constexpr int kSegThreads = 256;
 constexpr int kMaxK = 16;
 constexpr int kBg = -1;                        // parent entry of a background pixel
+constexpr int kBorderRoot = -2;                // cc_fill_holes: parent entry of a root whose component reaches the border
+
+// What cc_pack_kernel sets a bit for
+enum PackMode { kPackSet = 0 /* a non-zero byte */, kPackClearBytes = 1 /* a zero byte */,
+                kPackClearBits = 2 /* a clear bit of bit-packed planes with w % 32 == 0 */ };
 
 struct Plane {
     int h, w, n;          // n = h * w
@@ -84,13 +95,17 @@ __device__ __forceinline__ void unite(int* s, int a, int b) {
 }
 
 __global__ void __launch_bounds__(256) cc_pack_kernel(const uint8_t* __restrict__ mask, int n_planes, Plane g,
-                                                      uint32_t* __restrict__ bits) {
+                                                      int mode, uint32_t* __restrict__ bits) {
     const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
     const long long word = t >> 5;                       // one warp per word, one lane per pixel
     if (word >= static_cast<long long>(n_planes) * g.wpp) return;     // whole warps leave together
+    if (mode == kPackClearBits) {                        // same layout, no pad bits: the complement is ~word
+        if ((threadIdx.x & 31) == 0) bits[word] = ~__ldg(reinterpret_cast<const uint32_t*>(mask) + word);
+        return;
+    }
     const int p = static_cast<int>(word / g.wpp), wi = static_cast<int>(word - static_cast<long long>(p) * g.wpp);
     const int i = (wi << 5) + static_cast<int>(threadIdx.x & 31);
-    const bool on = i < g.n && mask[static_cast<size_t>(p) * g.n + i] != 0;
+    const bool on = i < g.n && (mask[static_cast<size_t>(p) * g.n + i] != 0) == (mode == kPackSet);
     const uint32_t v = __ballot_sync(0xffffffffu, on);
     if ((threadIdx.x & 31) == 0) bits[word] = v;
 }
@@ -366,6 +381,81 @@ unsigned long long work_words(int n_planes, const Plane& g) {
            (static_cast<unsigned long long>(g.n) + 5ull * g.cap + g.nseg + g.wpp);
 }
 
+Work work_of(void* workspace, int n_planes, const Plane& g) {
+    int* base = static_cast<int*>(workspace);
+    const size_t pn = static_cast<size_t>(n_planes) * g.n, pc = static_cast<size_t>(n_planes) * g.cap;
+    Work wk;
+    wk.parent = base;
+    wk.xmin = wk.parent + pn;
+    wk.xmax = wk.xmin + pc;
+    wk.ymin = wk.xmax + pc;
+    wk.ymax = wk.ymin + pc;
+    wk.count = wk.ymax + pc;
+    wk.seg = wk.count + pc;
+    wk.bits = reinterpret_cast<uint32_t*>(wk.seg + static_cast<size_t>(n_planes) * g.nseg);
+    return wk;
+}
+
+// Grid sizes of the labelling passes; false when one of them reaches 2^31 blocks or threads.
+struct Grids {
+    int tiles_x, tiles_per_plane;
+    long long merge_threads, seg_blocks, pack_blocks;
+};
+bool grids_of(int n_planes, const Plane& g, Grids* gr) {
+    gr->tiles_x = (g.w + kTileW - 1) / kTileW;
+    const long long tiles = static_cast<long long>(gr->tiles_x) * ((g.h + kTileH - 1) / kTileH);
+    gr->tiles_per_plane = static_cast<int>(tiles);
+    gr->merge_threads = tiles * n_planes * 64;
+    gr->seg_blocks = static_cast<long long>(n_planes) * g.nseg;
+    gr->pack_blocks = (static_cast<long long>(n_planes) * g.wpp * 32 + 255) / 256;
+    return tiles * n_planes < (1LL << 31) && static_cast<long long>(n_planes) * g.h < (1LL << 31) &&
+           gr->seg_blocks < (1LL << 31) && gr->pack_blocks < (1LL << 31);
+}
+
+// ---------------------------------------------------------------- hole filling (cc_fill_holes)
+// After cc_flatten_kernel over the complement, parent[i] is the root of background pixel i (kBg: a set pixel).
+// One thread per (plane, border position): the root of a background border pixel becomes kBorderRoot.  Only root
+// entries are written, all with the same value, and a non-root entry still names its root, so the order of the
+// writes does not matter.  Corner pixels come twice, which is harmless.
+__global__ void __launch_bounds__(256) cc_border_kernel(Plane g, long long n_threads, int* __restrict__ parent) {
+    const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (t >= n_threads) return;
+    const long long per = 2LL * (g.w + g.h), w = g.w;
+    const int p = static_cast<int>(t / per);
+    const long long k = t - p * per;
+    int x, y;
+    if (k < w) { x = static_cast<int>(k); y = 0; }
+    else if (k < 2 * w) { x = static_cast<int>(k - w); y = g.h - 1; }
+    else if (k < 2 * w + g.h) { x = 0; y = static_cast<int>(k - 2 * w); }
+    else { x = g.w - 1; y = static_cast<int>(k - 2 * w - g.h); }
+    int* par = parent + static_cast<size_t>(p) * g.n;
+    const int v = par[y * g.w + x];
+    if (v != kBg && v != kBorderRoot) par[v] = kBorderRoot;
+}
+
+// One warp per 32-pixel word (as cc_pack_kernel): a pixel is set when it is set in the input (kBg) or its
+// background component has an unmarked root.  Bit-packed output (w % 32 == 0) has the plane-contiguous word layout.
+__global__ void __launch_bounds__(256) cc_fill_kernel(Plane g, int n_planes, const int* __restrict__ parent,
+                                                      int out_packed, uint8_t* __restrict__ out) {
+    const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    const long long word = t >> 5;
+    if (word >= static_cast<long long>(n_planes) * g.wpp) return;     // whole warps leave together
+    const int p = static_cast<int>(word / g.wpp), wi = static_cast<int>(word - static_cast<long long>(p) * g.wpp);
+    const int i = (wi << 5) + static_cast<int>(threadIdx.x & 31);
+    const int* par = parent + static_cast<size_t>(p) * g.n;
+    bool on = false;
+    if (i < g.n) {
+        const int v = par[i];
+        on = v == kBg || (v != kBorderRoot && par[v] != kBorderRoot);
+    }
+    if (out_packed) {
+        const uint32_t b = __ballot_sync(0xffffffffu, on);
+        if ((threadIdx.x & 31) == 0) reinterpret_cast<uint32_t*>(out)[word] = b;
+    } else if (i < g.n) {
+        out[static_cast<size_t>(p) * g.n + i] = on ? 1 : 0;
+    }
+}
+
 // ---------------------------------------------------------------- oriented boxes of the selected components
 // (unetb200_mask_components_oriented): three more passes over the parent array after cc_select_kernel.
 //
@@ -635,37 +725,24 @@ int components_impl(const char* who, const uint8_t* mask, int packed, int n_plan
     } else if (workspace_bytes < 4ull * work_words(n_planes, g)) {
         return fail(UNETB200_ENOMEM, "workspace smaller than unetb200_components_workspace_bytes");
     }
-    const int tiles_x = (w + kTileW - 1) / kTileW, tiles_y = (h + kTileH - 1) / kTileH;
-    const long long tiles = static_cast<long long>(tiles_x) * tiles_y;
-    const long long n_rows = static_cast<long long>(n_planes) * h;
-    const long long seg_blocks = static_cast<long long>(n_planes) * g.nseg;
-    const long long pack_blocks = (static_cast<long long>(n_planes) * g.wpp * 32 + 255) / 256;
-    if (tiles * n_planes >= (1LL << 31) || n_rows >= (1LL << 31) || seg_blocks >= (1LL << 31) ||
-        pack_blocks >= (1LL << 31))
+    Grids gr;
+    if (!grids_of(n_planes, g, &gr))
         return fail(UNETB200_EINVAL, "batch too large");
-
-    int* base = static_cast<int*>(workspace);
-    const size_t pn = static_cast<size_t>(n_planes) * g.n, pc = static_cast<size_t>(n_planes) * g.cap;
-    Work wk;
-    wk.parent = base;
-    wk.xmin = wk.parent + pn;
-    wk.xmax = wk.xmin + pc;
-    wk.ymin = wk.xmax + pc;
-    wk.ymax = wk.ymin + pc;
-    wk.count = wk.ymax + pc;
-    wk.seg = wk.count + pc;
-    wk.bits = reinterpret_cast<uint32_t*>(wk.seg + static_cast<size_t>(n_planes) * g.nseg);
+    const int tiles_x = gr.tiles_x;
+    const long long n_rows = static_cast<long long>(n_planes) * h;
+    const long long seg_blocks = gr.seg_blocks;
+    const Work wk = work_of(workspace, n_planes, g);
 
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const uint32_t* bits = wk.bits;
     if (packed) {
         bits = reinterpret_cast<const uint32_t*>(mask);  // [h][w/8] with w % 32 == 0 is the plane-contiguous layout
     } else {
-        cc_pack_kernel<<<static_cast<unsigned>(pack_blocks), 256, 0, s>>>(mask, n_planes, g, wk.bits);
+        cc_pack_kernel<<<static_cast<unsigned>(gr.pack_blocks), 256, 0, s>>>(mask, n_planes, g, kPackSet, wk.bits);
     }
-    const int tpp = static_cast<int>(tiles);
-    const unsigned local_blocks = static_cast<unsigned>(tiles * n_planes);
-    const long long merge_threads = tiles * n_planes * 64;
+    const int tpp = gr.tiles_per_plane;
+    const unsigned local_blocks = static_cast<unsigned>(static_cast<long long>(tpp) * n_planes);
+    const long long merge_threads = gr.merge_threads;
     const unsigned merge_blocks = static_cast<unsigned>((merge_threads + 255) / 256);
     if (connectivity == 4) {
         cc_local_kernel<4><<<local_blocks, kTileW * kTileH, 0, s>>>(bits, g, tiles_x, tpp, wk.parent);
@@ -706,6 +783,39 @@ int components_impl(const char* who, const uint8_t* mask, int packed, int n_plan
 }
 
 }  // namespace
+
+int cc_fill_holes(const char* who, const uint8_t* in, int in_packed, uint8_t* out, int out_packed, int n_planes,
+                  int h, int w, void* workspace, cudaStream_t s) {
+    char buf[240];
+    Plane g;
+    Grids gr;
+    plane_of(h, w, &g);
+    const long long border_threads = static_cast<long long>(n_planes) * 2 * (static_cast<long long>(w) + h);
+    if (!grids_of(n_planes, g, &gr) || (border_threads + 255) / 256 >= (1LL << 31)) {
+        snprintf(buf, sizeof buf, "%s: batch too large", who);
+        return ub_fail(UNETB200_EINVAL, buf);
+    }
+    const Work wk = work_of(workspace, n_planes, g);
+    const unsigned pack_blocks = static_cast<unsigned>(gr.pack_blocks);
+    const unsigned local_blocks = static_cast<unsigned>(static_cast<long long>(gr.tiles_per_plane) * n_planes);
+    const unsigned merge_blocks = static_cast<unsigned>((gr.merge_threads + 255) / 256);
+    cc_pack_kernel<<<pack_blocks, 256, 0, s>>>(in, n_planes, g, in_packed ? kPackClearBits : kPackClearBytes,
+                                               wk.bits);
+    cc_local_kernel<4><<<local_blocks, kTileW * kTileH, 0, s>>>(wk.bits, g, gr.tiles_x, gr.tiles_per_plane,
+                                                                wk.parent);
+    cc_merge_kernel<4><<<merge_blocks, 256, 0, s>>>(wk.bits, g, gr.tiles_x, gr.tiles_per_plane, gr.merge_threads,
+                                                    wk.parent);
+    cc_flatten_kernel<<<static_cast<unsigned>(gr.seg_blocks), kSegThreads, 0, s>>>(g, wk.parent, wk.seg);
+    cc_border_kernel<<<static_cast<unsigned>((border_threads + 255) / 256), 256, 0, s>>>(g, border_threads,
+                                                                                        wk.parent);
+    cc_fill_kernel<<<pack_blocks, 256, 0, s>>>(g, n_planes, wk.parent, out_packed, out);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        snprintf(buf, sizeof buf, "%s: launch failed: %s", who, cudaGetErrorString(e));
+        return ub_fail(UNETB200_ECUDA, buf);
+    }
+    return UNETB200_OK;
+}
 
 extern "C" {
 

@@ -19,7 +19,8 @@ keeps working unmodified.  Differences, all internal:
 * ``run_unet_instances`` (new, additive) returns one crop per connected region of each field mask
   (``prepost.mask_components``) instead of one crop over all of its set pixels; with ``deskew=True`` each crop
   is cut upright along the region's principal axis (``prepost.mask_components_oriented`` +
-  ``prepost.warp_crops``), and ``enhance=True`` adds the OCR enhancement of each crop.
+  ``prepost.warp_crops``), and ``enhance=True`` adds the OCR enhancement of each crop; ``clean=`` cleans the
+  masks on the device (``prepost.mask_morphology`` / ``prepost.fill_holes``) before the regions are found.
 """
 from __future__ import annotations
 
@@ -526,7 +527,7 @@ def _segment_one(pil_img: Image.Image, checkpoint_path: str):
 
 
 def run_unet_instances(pil_img: Image.Image, checkpoint_path: str, max_instances: int = 4, min_pixels: int = 1,
-                       connectivity: int = 8, deskew: bool = False, enhance: bool = False):
+                       connectivity: int = 8, deskew: bool = False, enhance: bool = False, clean=None):
     """``run_unet`` with one crop per connected region of each field mask instead of one crop over all of its set
     pixels (new, additive; ``run_unet`` itself is unchanged).  Returns ``(masks, instances)``: ``masks`` exactly as
     ``run_unet`` returns them; ``instances[field]`` = list, largest region first, of ``{"box": (x1, y1, x2, y2),
@@ -541,27 +542,60 @@ def run_unet_instances(pil_img: Image.Image, checkpoint_path: str, max_instances
     each instance gains ``"quad"`` (the crop's four corners in the frame), ``"angle"`` (degrees, in (-90, 90]) and
     ``"size"`` (the region's length and width in frame pixels).  The near-black test applies to the upright crop.
     ``enhance=True`` adds ``"enhanced"``: the mode-"L" OCR enhancement (four times the crop size) of the crop, with
-    the field's ``ENHANCE_KINDS`` recipe, computed on the device from the crop's pixels there."""
+    the field's ``ENHANCE_KINDS`` recipe, computed on the device from the crop's pixels there.
+
+    ``clean``: steps applied in order to the masks on the device before the regions (and with ``deskew=True`` their
+    oriented boxes) are found; each is ``("open" | "close" | "erode" | "dilate", (kw, kh))`` (``cv2.morphologyEx``
+    with ``np.ones((kh, kw))``, kw, kh in 1..63) or ``"fill_holes"`` (``scipy.ndimage.binary_fill_holes``), e.g.
+    ``[("close", (9, 3)), "fill_holes", ("open", (3, 3))]``.  The returned ``masks`` stay ``run_unet``'s, uncleaned.
+    A malformed step raises ``ValueError`` before any GPU work."""
     from . import prepost
+    steps = _clean_steps(clean)
     frame, mask = _segment_one(pil_img, checkpoint_path)
-    m_cpu = None
+    m_cpu = mask[0].cpu().numpy()
+    packed = False
+    for op, ks in steps:                               # bit-packed between and after the steps (W = 512)
+        if op == "fill_holes":
+            mask = prepost.fill_holes(mask, packed=packed, out_packed=True)
+        else:
+            mask = prepost.mask_morphology(mask, op, ks, packed=packed, out_packed=True)
+        packed = True
     if not deskew:
-        comps, _ = prepost.mask_components(mask, connectivity=connectivity, max_components=max_instances)
-        m_cpu = mask[0].cpu().numpy()
+        comps, _ = prepost.mask_components(mask, packed=packed, connectivity=connectivity,
+                                           max_components=max_instances)
         inst = components_to_instances(pil_img, comps[0].cpu().numpy(), frame, min_pixels)
         if enhance:
             _enhance_instances(inst, frame)
     else:
         scale = (pil_img.size[0] / IMG_SIZE, pil_img.size[1] / IMG_SIZE)
-        comps, _, _, obox = prepost.mask_components_oriented(mask, connectivity=connectivity,
+        comps, _, _, obox = prepost.mask_components_oriented(mask, packed=packed, connectivity=connectivity,
                                                              max_components=max_instances, scale=scale)
-        m_cpu = mask[0].cpu().numpy()
         if frame is None:                              # other PIL modes: the RGB conversion goes up for the warp
             frame = _upload_rgb(pil_img.convert("RGB"))[0]
         inst = _deskewed_instances(pil_img, comps[0].cpu().numpy(), obox[0].cpu().numpy(), frame, scale,
                                    min_pixels, enhance)
     masks = {f: m_cpu[i] != 0 for i, f in enumerate(FIELDS)}
     return masks, inst
+
+
+def _clean_steps(clean) -> List[Tuple[str, Optional[Tuple[int, int]]]]:
+    """``clean`` of :func:`run_unet_instances` -> ``[(op, (kw, kh) or None), ...]``, else ``ValueError``."""
+    from . import prepost
+    if clean is None:
+        return []
+    if isinstance(clean, (str, bytes)) or not isinstance(clean, Sequence):
+        raise ValueError(f"clean must be a sequence of steps; got {clean!r}")
+    steps = []
+    for step in clean:
+        if isinstance(step, str) and step == "fill_holes":
+            steps.append(("fill_holes", None))
+        elif (isinstance(step, (tuple, list)) and len(step) == 2 and isinstance(step[0], str)
+              and step[0] in prepost.MORPH_OPS):
+            steps.append((step[0], prepost._ksize(step[1])))
+        else:
+            raise ValueError(f"clean step must be (\"open\" | \"close\" | \"erode\" | \"dilate\", (kw, kh)) or "
+                             f"\"fill_holes\"; got {step!r}")
+    return steps
 
 
 def _deskewed_instances(pil_img: Image.Image, comps: np.ndarray, obox: np.ndarray, frame_dev: torch.Tensor, scale,

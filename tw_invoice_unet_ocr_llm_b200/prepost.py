@@ -8,6 +8,8 @@
   of the largest regions of each plane), where ``mask_bbox`` gives one box over all set pixels;
 * ``mask_components_oriented`` -- the same plus the moments and the oriented box (principal axis and extents in
   frame coordinates) of every listed region;
+* ``mask_morphology`` / ``fill_holes`` -- erosion, dilation, opening and closing of the masks by a rectangle
+  (``cv2.erode`` / ``cv2.dilate`` / ``cv2.morphologyEx``) and ``scipy.ndimage.binary_fill_holes``, bit for bit;
 * ``warp_crops`` -- a ragged batch of affine crops of device frames, bit-identical to ``cv2.warpAffine``
   (``INTER_LINEAR | WARP_INVERSE_MAP``, ``BORDER_REPLICATE``), with the byte sum of each crop.
 """
@@ -150,6 +152,71 @@ def mask_components(mask: torch.Tensor, *, packed: bool = False, connectivity: i
             None if lab is None else lab.data_ptr(), comps.data_ptr(), counts.data_ptr(), ws.data_ptr(), ws_bytes,
             torch.cuda.current_stream(dev).cuda_stream))
     return (comps, counts, lab) if labels else (comps, counts)
+
+
+MORPH_OPS = {"erode": nat.MORPH_ERODE, "dilate": nat.MORPH_DILATE, "open": nat.MORPH_OPEN, "close": nat.MORPH_CLOSE}
+
+
+def _morph(name: str, mask: torch.Tensor, op: int, kw: int, kh: int, packed: bool, out_packed, out):
+    if mask.dtype != torch.uint8 or mask.dim() != 4 or not mask.is_cuda:
+        raise RuntimeError(f"{name} expects a CUDA uint8 [N,C,H,W] (or [N,C,H,W/8] bit-packed) tensor")
+    mask = mask.contiguous()
+    n, c, h, wm = mask.shape
+    w = wm * 8 if packed else wm
+    out_packed = bool(packed) if out_packed is None else bool(out_packed)
+    shape = (n, c, h, w // 8 if out_packed else w)
+    dev = mask.device
+    if out is None:
+        out = torch.empty(shape, dtype=torch.uint8, device=dev)
+    elif out.dtype != torch.uint8 or tuple(out.shape) != shape or out.device != dev or not out.is_contiguous():
+        raise RuntimeError(f"{name}: out must be a contiguous uint8 {list(shape)} tensor on the same device")
+    lib = nat.lib()
+    ws_bytes = lib.unetb200_morph_workspace_bytes(n * c, h, w, op)
+    if ws_bytes == 0:
+        raise RuntimeError(f"{name}: bad mask shape {tuple(mask.shape)}")
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        nat.check(lib.unetb200_mask_morph(mask.data_ptr(), int(bool(packed)), out.data_ptr(), int(out_packed), n * c,
+                                          h, w, op, kw, kh, ws.data_ptr(), ws_bytes,
+                                          torch.cuda.current_stream(dev).cuda_stream))
+    return out
+
+
+def mask_morphology(mask: torch.Tensor, op: str, ksize=(3, 3), *, packed: bool = False, out_packed: bool = None,
+                    out: torch.Tensor = None) -> torch.Tensor:
+    """Erosion, dilation, opening or closing (``op`` = ``"erode"``, ``"dilate"``, ``"open"``, ``"close"``) of every
+    plane of uint8 ``[N, C, H, W]`` masks (non-zero = set), or of bit-packed ``[N, C, H, W/8]`` masks with
+    ``packed=True`` (``Engine.run(mask_bits=True)``; ``W`` a multiple of 32), by a ``ksize = (kw, kh)`` rectangle
+    (1..63 each).  Equal to ``cv2.erode`` / ``cv2.dilate`` / ``cv2.morphologyEx(MORPH_OPEN / MORPH_CLOSE)`` with
+    ``np.ones((kh, kw))``, the default anchor and the default border (pixels outside the plane take no part).
+
+    Returns 0 / 1 bytes ``[N, C, H, W]``, or bit-packed ``[N, C, H, W/8]`` with ``out_packed=True`` (default: as the
+    input).  ``out``: optional contiguous destination of that shape; the input itself is allowed (in place).
+    Enqueued on the current stream."""
+    if op not in MORPH_OPS:
+        raise ValueError(f"mask_morphology: op must be one of {sorted(MORPH_OPS)}; got {op!r}")
+    kw, kh = _ksize(ksize)
+    return _morph("mask_morphology", mask, MORPH_OPS[op], kw, kh, packed, out_packed, out)
+
+
+def fill_holes(mask: torch.Tensor, *, packed: bool = False, out_packed: bool = None,
+               out: torch.Tensor = None) -> torch.Tensor:
+    """``scipy.ndimage.binary_fill_holes`` of every plane (default structure: a hole is a 4-connected background
+    region that touches no border pixel).  Input, output and ``out`` as :func:`mask_morphology`.  Enqueued on the
+    current stream."""
+    return _morph("fill_holes", mask, nat.MORPH_FILL_HOLES, 0, 0, packed, out_packed, out)
+
+
+def _ksize(ksize):
+    """``(kw, kh)`` of two ints in 1..63, else ``ValueError``."""
+    try:
+        kw, kh = ksize
+    except (TypeError, ValueError):
+        raise ValueError(f"ksize must be (kw, kh); got {ksize!r}") from None
+    for v in (kw, kh):
+        if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or not 1 <= v <= 63:
+            raise ValueError(f"ksize must be two ints in 1..63; got {ksize!r}")
+    return int(kw), int(kh)
 
 
 def _plane_scale(scale, n: int, c: int, dev) -> torch.Tensor:
