@@ -306,6 +306,32 @@ uint64_t unetb200_morph_workspace_bytes(int n_planes, int h, int w, int op);
  * a short workspace UNETB200_ENOMEM. */
 int unetb200_mask_morph(const uint8_t* in, int in_packed, uint8_t* out, int out_packed, int n_planes, int h, int w,
                         int op, int kw, int kh, void* workspace, uint64_t workspace_bytes, void* stream);
+/* Scores predicted planes against ground-truth planes (DESIGN.md 6b, "Region matching"; oracle/mask_match.py):
+ *   pred, gt   byte planes uint8 [n_planes, h, w] (non-zero = set) or, with pred_packed / gt_packed = 1, bit-packed
+ *              planes uint8 [n_planes, h, w/8] in the format of unetb200_forward_bits (w % 32 == 0, 4-byte aligned);
+ *              any of the four combinations; h, w >= 1, h * w < 2^31 as unetb200_mask_components
+ *   regions    the connected components of each plane (connectivity 4 or 8, the labels of unetb200_mask_components);
+ *              a pred region with fewer than min_pixels (>= 1) pixels is ignored, gt regions never are
+ *   match      pred region a and gt region g match when I > t (x) U, I = |a n g| and U = |a| + |g| - I exact
+ *              integers and (x) one correctly rounded float64 product; t = iou_threshold in [0.5, 1), so a region
+ *              has at most one partner
+ *   counts     int64 [n_planes, 8] = px_tp, px_fp, px_fn (set/set, set/clear, clear/set pixels, all of them),
+ *              n_pred (pred regions of >= min_pixels pixels), n_gt (gt regions), tp (matched pairs), sum of I and
+ *              sum of U over the matched pairs
+ *   iou_sum    float64 [n_planes]: sum of the correctly rounded I / U over the matched pairs; thread j of 256 adds the
+ *              pairs of pred labels j + 1, j + 257, ... in ascending order from +0.0, then s[j] += s[j + half] for
+ *              half = 128, 64, ..., 1 combines the partial sums
+ *   workspace  >= unetb200_match_workspace_bytes(n_planes, h, w) bytes, 16-byte aligned, no initialisation: two
+ *              components workspaces (each rounded up to 16 bytes), 12 bytes per statistics row (ceil(h * w / 2)
+ *              rows per plane) and 8 bytes per plane
+ * counts and iou_sum are 8-byte aligned.  Deterministic bits.  Asynchronous: enqueued on `stream`, nothing is
+ * allocated.  A null pointer, a bad size, flag, connectivity, min_pixels or threshold (not finite or outside
+ * [0.5, 1)), or a misaligned pointer is UNETB200_EINVAL; a short workspace UNETB200_ENOMEM.  The query returns 0 for
+ * a bad size. */
+uint64_t unetb200_match_workspace_bytes(int n_planes, int h, int w);
+int unetb200_mask_match(const uint8_t* pred, int pred_packed, const uint8_t* gt, int gt_packed, int n_planes, int h,
+                        int w, int connectivity, int min_pixels, double iou_threshold, int64_t* counts,
+                        double* iou_sum, void* workspace, uint64_t workspace_bytes, void* stream);
 /* Ragged batch of affine crops: output pixel (j, i) of crop k samples its frame at (m0 j + m1 i + m2, m3 j + m4 i + m5),
  * bilinear with replicated borders, bit-identical to cv2.warpAffine(src, M, (out_w, out_h),
  * flags=INTER_LINEAR | WARP_INVERSE_MAP, borderMode=BORDER_REPLICATE) of the RGB frame. */

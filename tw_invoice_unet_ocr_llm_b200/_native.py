@@ -107,6 +107,8 @@ SYMBOLS = {
                                                _U64, _VP]),
     "unetb200_morph_workspace_bytes": (_U64, [_I, _I, _I, _I]),
     "unetb200_mask_morph": (_I, [_VP, _I, _VP, _I, _I, _I, _I, _I, _I, _I, _VP, _U64, _VP]),
+    "unetb200_match_workspace_bytes": (_U64, [_I, _I, _I]),
+    "unetb200_mask_match": (_I, [_VP, _I, _VP, _I, _I, _I, _I, _I, _I, C.c_double, _VP, _VP, _VP, _U64, _VP]),
     "unetb200_warp_crops": (_I, [C.POINTER(WarpCrop), _VP, _I, _VP, _VP, _VP]),
     "unetb200_box_sums": (_I, [_VP, _I, _I, _I, C.POINTER(C.c_int32), _I, _VP, _VP]),
     "unetb200_box_sums_ps": (_I, [_VP, _I, _I, _I, _I, C.POINTER(C.c_int32), _I, _VP, _VP]),

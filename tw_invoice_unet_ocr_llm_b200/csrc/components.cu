@@ -23,6 +23,9 @@
 // same union-find: cc_pack_kernel in a complement mode, cc_local / cc_merge (4-connectivity) and cc_flatten, then
 // cc_border_kernel marks the roots of the components that reach the border and cc_fill_kernel writes the planes
 // with every unmarked background component set.
+//
+// cc_label (unetb200_mask_match, csrc/match.cu) runs the passes pack .. stats without the selection, so the
+// workspace keeps the pixel -> component map and the size of every component of a plane.
 #include "../../include/unetb200.h"
 
 #include <cuda_runtime.h>
@@ -412,6 +415,38 @@ bool grids_of(int n_planes, const Plane& g, Grids* gr) {
            gr->seg_blocks < (1LL << 31) && gr->pack_blocks < (1LL << 31);
 }
 
+// The labelling passes pack .. stats: afterwards parent[i] names the component of pixel i (cc_pixel_id),
+// count[id] is the size of every component and n_comps[plane] their number.  Sizes already validated, grids
+// checked by grids_of.
+void label_passes(const uint8_t* mask, int packed, int n_planes, const Plane& g, const Grids& gr, int connectivity,
+                  const Work& wk, int32_t* labels, int32_t* n_comps, cudaStream_t s) {
+    const int tiles_x = gr.tiles_x;
+    const long long n_rows = static_cast<long long>(n_planes) * g.h;
+    const long long seg_blocks = gr.seg_blocks;
+    const uint32_t* bits = wk.bits;
+    if (packed) {
+        bits = reinterpret_cast<const uint32_t*>(mask);  // [h][w/8] with w % 32 == 0 is the plane-contiguous layout
+    } else {
+        cc_pack_kernel<<<static_cast<unsigned>(gr.pack_blocks), 256, 0, s>>>(mask, n_planes, g, kPackSet, wk.bits);
+    }
+    const int tpp = gr.tiles_per_plane;
+    const unsigned local_blocks = static_cast<unsigned>(static_cast<long long>(tpp) * n_planes);
+    const long long merge_threads = gr.merge_threads;
+    const unsigned merge_blocks = static_cast<unsigned>((merge_threads + 255) / 256);
+    if (connectivity == 4) {
+        cc_local_kernel<4><<<local_blocks, kTileW * kTileH, 0, s>>>(bits, g, tiles_x, tpp, wk.parent);
+        cc_merge_kernel<4><<<merge_blocks, 256, 0, s>>>(bits, g, tiles_x, tpp, merge_threads, wk.parent);
+    } else {
+        cc_local_kernel<8><<<local_blocks, kTileW * kTileH, 0, s>>>(bits, g, tiles_x, tpp, wk.parent);
+        cc_merge_kernel<8><<<merge_blocks, 256, 0, s>>>(bits, g, tiles_x, tpp, merge_threads, wk.parent);
+    }
+    cc_flatten_kernel<<<static_cast<unsigned>(seg_blocks), kSegThreads, 0, s>>>(g, wk.parent, wk.seg);
+    cc_scan_kernel<<<static_cast<unsigned>(n_planes), 1024, 0, s>>>(g, wk.seg, n_comps);
+    cc_number_kernel<<<static_cast<unsigned>(seg_blocks), kSegThreads, 0, s>>>(g, wk.parent, wk.seg, wk);
+    cc_stats_kernel<<<static_cast<unsigned>((n_rows + 7) / 8), 256, 0, s>>>(g, static_cast<int>(n_rows), wk.parent,
+                                                                            wk, labels);
+}
+
 // ---------------------------------------------------------------- hole filling (cc_fill_holes)
 // After cc_flatten_kernel over the complement, parent[i] is the root of background pixel i (kBg: a set pixel).
 // One thread per (plane, border position): the root of a background border pixel becomes kBorderRoot.  Only root
@@ -477,13 +512,6 @@ unsigned long long oriented_bytes(int n_planes, const Plane& g) {
     return oriented_tail_offset(n_planes, g) + static_cast<unsigned long long>(n_planes) * kMaxK * 4 * 8;
 }
 
-// Component id of pixel i (-1 = background), as cc_stats_kernel reads it after cc_number_kernel.
-__device__ __forceinline__ int pixel_id(const int* __restrict__ par, int i) {
-    const int v = par[i];
-    if (v == kBg) return -1;
-    return v < kBg ? -v - 2 : -par[v] - 2;
-}
-
 // Row of the plane's selection that holds component `id`, or -1 (ids are unique within a plane).
 __device__ __forceinline__ int slot_of(const int* sel, int k_out, int id) {
     int s = -1;
@@ -528,7 +556,7 @@ __global__ void __launch_bounds__(256) cc_moments_kernel(Plane g, const int* __r
     const uint32_t bit[5] = {0xaaaaaaaau, 0xccccccccu, 0xf0f0f0f0u, 0xff00ff00u, 0xffff0000u};   // bit j of lane index
     for (int x0 = 0; x0 < g.w; x0 += 32) {
         const int x = x0 + lane;
-        const int slot = x < g.w ? slot_of(sel, k_out, pixel_id(par, y * g.w + x)) : -1;
+        const int slot = x < g.w ? slot_of(sel, k_out, cc_pixel_id(par, y * g.w + x)) : -1;
         const uint32_t grp = __match_any_sync(0xffffffffu, slot);
         if (slot >= 0 && lane == __ffs(grp) - 1) {
             long long s1 = 0, s2 = 0;
@@ -649,7 +677,7 @@ __global__ void __launch_bounds__(256) cc_extent_kernel(Plane g, const int* __re
     long long* kp = keys + static_cast<size_t>(p) * k_out * 4;
     for (int x0 = 0; x0 < g.w; x0 += 32) {
         const int x = x0 + lane;
-        const int slot = x < g.w ? slot_of(sel, k_out, pixel_id(par, y * g.w + x)) : -1;
+        const int slot = x < g.w ? slot_of(sel, k_out, cc_pixel_id(par, y * g.w + x)) : -1;
         const uint32_t grp = __match_any_sync(0xffffffffu, slot);
         if (slot >= 0 && lane == __ffs(grp) - 1) {
             double u0, v0, u1, v1;
@@ -728,34 +756,9 @@ int components_impl(const char* who, const uint8_t* mask, int packed, int n_plan
     Grids gr;
     if (!grids_of(n_planes, g, &gr))
         return fail(UNETB200_EINVAL, "batch too large");
-    const int tiles_x = gr.tiles_x;
-    const long long n_rows = static_cast<long long>(n_planes) * h;
-    const long long seg_blocks = gr.seg_blocks;
     const Work wk = work_of(workspace, n_planes, g);
-
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    const uint32_t* bits = wk.bits;
-    if (packed) {
-        bits = reinterpret_cast<const uint32_t*>(mask);  // [h][w/8] with w % 32 == 0 is the plane-contiguous layout
-    } else {
-        cc_pack_kernel<<<static_cast<unsigned>(gr.pack_blocks), 256, 0, s>>>(mask, n_planes, g, kPackSet, wk.bits);
-    }
-    const int tpp = gr.tiles_per_plane;
-    const unsigned local_blocks = static_cast<unsigned>(static_cast<long long>(tpp) * n_planes);
-    const long long merge_threads = gr.merge_threads;
-    const unsigned merge_blocks = static_cast<unsigned>((merge_threads + 255) / 256);
-    if (connectivity == 4) {
-        cc_local_kernel<4><<<local_blocks, kTileW * kTileH, 0, s>>>(bits, g, tiles_x, tpp, wk.parent);
-        cc_merge_kernel<4><<<merge_blocks, 256, 0, s>>>(bits, g, tiles_x, tpp, merge_threads, wk.parent);
-    } else {
-        cc_local_kernel<8><<<local_blocks, kTileW * kTileH, 0, s>>>(bits, g, tiles_x, tpp, wk.parent);
-        cc_merge_kernel<8><<<merge_blocks, 256, 0, s>>>(bits, g, tiles_x, tpp, merge_threads, wk.parent);
-    }
-    cc_flatten_kernel<<<static_cast<unsigned>(seg_blocks), kSegThreads, 0, s>>>(g, wk.parent, wk.seg);
-    cc_scan_kernel<<<static_cast<unsigned>(n_planes), 1024, 0, s>>>(g, wk.seg, n_comps);
-    cc_number_kernel<<<static_cast<unsigned>(seg_blocks), kSegThreads, 0, s>>>(g, wk.parent, wk.seg, wk);
-    cc_stats_kernel<<<static_cast<unsigned>((n_rows + 7) / 8), 256, 0, s>>>(g, static_cast<int>(n_rows), wk.parent,
-                                                                            wk, labels);
+    label_passes(mask, packed, n_planes, g, gr, connectivity, wk, labels, n_comps, s);
     cc_select_kernel<<<static_cast<unsigned>(n_planes), 256, 0, s>>>(g, wk, n_comps, max_components, comps);
     if (ori) {
         const int k = max_components, rows = n_planes * k;
@@ -809,6 +812,34 @@ int cc_fill_holes(const char* who, const uint8_t* in, int in_packed, uint8_t* ou
     cc_border_kernel<<<static_cast<unsigned>((border_threads + 255) / 256), 256, 0, s>>>(g, border_threads,
                                                                                         wk.parent);
     cc_fill_kernel<<<pack_blocks, 256, 0, s>>>(g, n_planes, wk.parent, out_packed, out);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        snprintf(buf, sizeof buf, "%s: launch failed: %s", who, cudaGetErrorString(e));
+        return ub_fail(UNETB200_ECUDA, buf);
+    }
+    return UNETB200_OK;
+}
+
+bool cc_batch_fits(int n_planes, int h, int w) {
+    Plane g;
+    Grids gr;
+    return n_planes > 0 && plane_of(h, w, &g) && grids_of(n_planes, g, &gr);
+}
+
+int cc_label(const char* who, const uint8_t* mask, int packed, int n_planes, int h, int w, int connectivity,
+             void* workspace, int32_t* n_comps, cudaStream_t s, CcLabels* out) {
+    char buf[240];
+    Plane g;
+    Grids gr;
+    if (n_planes <= 0 || !plane_of(h, w, &g) || !grids_of(n_planes, g, &gr)) {
+        snprintf(buf, sizeof buf, "%s: batch too large", who);
+        return ub_fail(UNETB200_EINVAL, buf);
+    }
+    const Work wk = work_of(workspace, n_planes, g);
+    label_passes(mask, packed, n_planes, g, gr, connectivity, wk, nullptr, n_comps, s);
+    out->parent = wk.parent;
+    out->count = wk.count;
+    out->cap = g.cap;
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {
         snprintf(buf, sizeof buf, "%s: launch failed: %s", who, cudaGetErrorString(e));

@@ -598,6 +598,85 @@ def _clean_steps(clean) -> List[Tuple[str, Optional[Tuple[int, int]]]]:
     return steps
 
 
+def evaluate_masks(model, x: torch.Tensor, gt: torch.Tensor, *, thresholds=None, clean=None, connectivity: int = 8,
+                   min_pixels: int = 1, iou: float = 0.5) -> Dict[str, dict]:
+    """Scores the field masks of ``model`` on ``x`` against the ground-truth masks ``gt`` (new, additive): the number
+    for choosing ``thresholds``, ``clean``, ``min_pixels`` and ``connectivity`` on a validation set.
+
+    ``model``: a ``UNet`` (its current weights) or a checkpoint path.  ``x``: any input of the eval forward
+    (float32 / float16 / bfloat16 ``[N, 3, H, W]``, uint8 ``[N, H, W, 3]``), ``gt``: ``[N, 3, H, W]`` in ``FIELDS``
+    order, non-zero = set; tensors on the host are moved to the device chunk by chunk.  ``thresholds``: per-field
+    sigmoid thresholds (a dict over ``FIELDS`` or three numbers; default ``THRESHOLDS``).  ``clean``: the clean-up
+    steps of :func:`run_unet_instances`, applied on the device before scoring (a malformed step raises
+    ``ValueError`` before any GPU work).  Regions, ``min_pixels`` (pred regions only) and the IoU rule
+    (``0.5 <= iou < 1``) are those of ``prepost.mask_match``.
+
+    Chunks of ``MAX_CHUNK`` images run forward (bit-packed masks when ``W % 32 == 0``), clean-up and matching on the
+    device; the counts accumulate there and come back in one copy.  Returns ``{field: dict}`` with the summed counts
+    (``prepost.MATCH_COUNTS`` and ``iou_sum``, added with ``math.fsum``) and the metrics, ``None`` where a
+    denominator is 0: ``pixel_iou``, ``dice``, ``pixel_precision`` and ``pixel_recall`` over pixels; ``precision``
+    (``tp / n_pred``), ``recall`` (``tp / n_gt``) and ``f1`` over regions; panoptic ``sq = iou_sum / tp``,
+    ``rq = tp / (tp + fp / 2 + fn / 2)`` and ``pq = iou_sum / (tp + fp / 2 + fn / 2)`` with ``fp = n_pred - tp``,
+    ``fn = n_gt - tp``."""
+    from . import prepost
+    steps = _clean_steps(clean)
+    if thresholds is None:
+        thresholds = THRESHOLDS
+    thr = [float(thresholds[f]) for f in FIELDS] if isinstance(thresholds, dict) else [float(t) for t in thresholds]
+    if len(thr) != len(FIELDS):
+        raise ValueError(f"thresholds: one per field of {FIELDS}; got {thresholds!r}")
+    if isinstance(model, UNet):
+        _require_cuda()
+        eng = model.engine(x.device if x.is_cuda else DEVICE)
+    else:
+        _require_cuda()
+        _, eng = _cached_engine(model)
+    dev = eng.device
+    n = x.shape[0]
+    h, w = (x.shape[1], x.shape[2]) if x.dtype == torch.uint8 else (x.shape[2], x.shape[3])
+    if gt.dim() != 4 or tuple(gt.shape) != (n, len(FIELDS), h, w):
+        raise ValueError(f"gt must be [N, {len(FIELDS)}, H, W] = {(n, len(FIELDS), h, w)}; got {tuple(gt.shape)}")
+    packed = w % 32 == 0
+    counts = torch.zeros((len(FIELDS), 8), dtype=torch.int64, device=dev)
+    sums = torch.empty((n, len(FIELDS)), dtype=torch.float64, device=dev)
+    for lo in range(0, n, MAX_CHUNK):
+        hi = min(n, lo + MAX_CHUNK)
+        xc = x[lo:hi].to(dev)
+        g = gt[lo:hi].to(dev)
+        g = g if g.dtype == torch.uint8 else (g != 0).to(torch.uint8)
+        _, mask = eng.run(xc, want_logits=False, thresholds=thr, mask_bits=packed)
+        for op, ks in steps:
+            if op == "fill_holes":
+                prepost.fill_holes(mask, packed=packed, out=mask)
+            else:
+                prepost.mask_morphology(mask, op, ks, packed=packed, out=mask)
+        c, s = prepost.mask_match(mask, g, pred_packed=packed, connectivity=connectivity, min_pixels=min_pixels,
+                                  iou=iou)
+        counts += c.sum(dim=0)
+        sums[lo:hi] = s
+    # one copy back: the int64 counts travel as their float64 bit patterns next to the per-plane sums
+    host = torch.cat([counts.view(-1).view(torch.float64), sums.view(-1)]).cpu()
+    tot = host[:counts.numel()].view(torch.int64).view(len(FIELDS), 8).tolist()
+    per_plane = host[counts.numel():].view(n, len(FIELDS)).numpy()
+    return {f: _match_metrics(dict(zip(prepost.MATCH_COUNTS, tot[i])), math.fsum(per_plane[:, i].tolist()))
+            for i, f in enumerate(FIELDS)}
+
+
+def _match_metrics(c: dict, iou_sum: float) -> dict:
+    """Summed counts of ``prepost.mask_match`` -> the counts, ``iou_sum`` and the metrics of :func:`evaluate_masks`."""
+    def ratio(num, den):
+        return None if den == 0 else num / den
+    tp, fp, fn = c["px_tp"], c["px_fp"], c["px_fn"]
+    rtp, rfp, rfn = c["tp"], c["n_pred"] - c["tp"], c["n_gt"] - c["tp"]
+    out = dict(c, iou_sum=iou_sum)
+    out.update(pixel_iou=ratio(tp, tp + fp + fn), dice=ratio(2 * tp, 2 * tp + fp + fn),
+               pixel_precision=ratio(tp, tp + fp), pixel_recall=ratio(tp, tp + fn),
+               precision=ratio(rtp, c["n_pred"]), recall=ratio(rtp, c["n_gt"]),
+               f1=ratio(2 * rtp, c["n_pred"] + c["n_gt"]), sq=ratio(iou_sum, rtp),
+               rq=ratio(rtp, rtp + 0.5 * rfp + 0.5 * rfn), pq=ratio(iou_sum, rtp + 0.5 * rfp + 0.5 * rfn))
+    return out
+
+
 def _deskewed_instances(pil_img: Image.Image, comps: np.ndarray, obox: np.ndarray, frame_dev: torch.Tensor, scale,
                         min_pixels: int, enhance: bool) -> Dict[str, List[dict]]:
     """Rows of ``prepost.mask_components_oriented`` for one image -> instances with upright crops: the rows

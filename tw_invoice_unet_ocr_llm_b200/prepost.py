@@ -10,6 +10,8 @@
   frame coordinates) of every listed region;
 * ``mask_morphology`` / ``fill_holes`` -- erosion, dilation, opening and closing of the masks by a rectangle
   (``cv2.erode`` / ``cv2.dilate`` / ``cv2.morphologyEx``) and ``scipy.ndimage.binary_fill_holes``, bit for bit;
+* ``mask_match`` -- predicted masks scored against ground truth: pixel counts and the one-to-one matching of their
+  regions at IoU > t;
 * ``warp_crops`` -- a ragged batch of affine crops of device frames, bit-identical to ``cv2.warpAffine``
   (``INTER_LINEAR | WARP_INVERSE_MAP``, ``BORDER_REPLICATE``), with the byte sum of each crop.
 """
@@ -217,6 +219,51 @@ def _ksize(ksize):
         if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or not 1 <= v <= 63:
             raise ValueError(f"ksize must be two ints in 1..63; got {ksize!r}")
     return int(kw), int(kh)
+
+
+MATCH_COUNTS = ("px_tp", "px_fp", "px_fn", "n_pred", "n_gt", "tp", "sum_inter", "sum_union")
+
+
+def mask_match(pred: torch.Tensor, gt: torch.Tensor, *, pred_packed: bool = False, gt_packed: bool = False,
+               connectivity: int = 8, min_pixels: int = 1, iou: float = 0.5):
+    """Scores predicted masks against ground truth, plane by plane (DESIGN.md 6b, "Region matching").
+
+    ``pred`` and ``gt``: uint8 ``[N, C, H, W]`` (non-zero = set), or bit-packed ``[N, C, H, W/8]`` with
+    ``pred_packed`` / ``gt_packed`` (``Engine.run(mask_bits=True)``; ``W`` a multiple of 32), on one CUDA device.
+    Regions are the connected components of each plane (``connectivity`` 4 or 8, as :func:`mask_components`); a pred
+    region of fewer than ``min_pixels`` pixels is ignored.  A pred region ``a`` and a gt region ``g`` match when
+    ``I > iou * U`` (``I = |a & g|``, ``U = |a| + |g| - I``, one float64 product), ``0.5 <= iou < 1``: each region has
+    at most one partner.
+
+    Returns ``(counts, iou_sum)``: int64 ``[N, C, 8]`` = :data:`MATCH_COUNTS` (pixel true positives, false
+    positives, false negatives; pred regions kept, gt regions; matched pairs and the sums of their I and U) and
+    float64 ``[N, C]`` = the sum of ``I / U`` over the matched pairs, in a fixed order (``oracle/mask_match.py``).
+    Enqueued on the current stream."""
+    for name, t in (("pred", pred), ("gt", gt)):
+        if t.dtype != torch.uint8 or t.dim() != 4 or not t.is_cuda:
+            raise RuntimeError(f"mask_match expects {name} as a CUDA uint8 [N,C,H,W] (or [N,C,H,W/8] bit-packed) "
+                               "tensor")
+    pred, gt = pred.contiguous(), gt.contiguous()
+    n, c, h, wp = pred.shape
+    w = wp * 8 if pred_packed else wp
+    gw = gt.shape[3] * 8 if gt_packed else gt.shape[3]
+    if tuple(gt.shape[:3]) != (n, c, h) or gw != w or gt.device != pred.device:
+        raise RuntimeError(f"mask_match: pred {tuple(pred.shape)} (packed={bool(pred_packed)}) and gt "
+                           f"{tuple(gt.shape)} (packed={bool(gt_packed)}) are not planes of one shape on one device")
+    lib = nat.lib()
+    ws_bytes = lib.unetb200_match_workspace_bytes(n * c, h, w)
+    if ws_bytes == 0:
+        raise RuntimeError(f"mask_match: bad mask shape {tuple(pred.shape)}")
+    dev = pred.device
+    counts = torch.empty((n, c, 8), dtype=torch.int64, device=dev)
+    iou_sum = torch.empty((n, c), dtype=torch.float64, device=dev)
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        nat.check(lib.unetb200_mask_match(
+            pred.data_ptr(), int(bool(pred_packed)), gt.data_ptr(), int(bool(gt_packed)), n * c, h, w,
+            int(connectivity), int(min_pixels), float(iou), counts.data_ptr(), iou_sum.data_ptr(), ws.data_ptr(),
+            ws_bytes, torch.cuda.current_stream(dev).cuda_stream))
+    return counts, iou_sum
 
 
 def _plane_scale(scale, n: int, c: int, dev) -> torch.Tensor:
