@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define UNETB200_ABI_VERSION 1
+#define UNETB200_ABI_VERSION 2
 
 enum {
     UNETB200_OK = 0,
@@ -377,8 +377,13 @@ uint32_t unetb200_test_fastdiv(uint32_t d, uint32_t x);
 typedef struct unetb200_enh_crop {
     int32_t h, w;             /* in : crop size in pixels (output is 4h x 4w) */
     int32_t flags;            /* in : UNETB200_ENH_* */
-    float clip;               /* in : CLAHE clipLimit (> 0) */
-    int32_t clip_count;       /* out: per-bin clip limit, max((int)(clip * tile_area / 256), 1) */
+    double clip;              /* in : CLAHE clipLimit, finite and > 0; a double, as cv::createCLAHE takes it
+                               *      (4 bytes of alignment padding precede it) */
+    int32_t clip_count;       /* out: per-bin clip limit, max((int)min(clip * tile_area / 256, tile_area), 1) in
+                               *      double: OpenCV's (int)(clipLimit * tileSizeTotal / 256), clamped at the tile
+                               *      area.  No bin holds more than the area, so a limit at or above it clips
+                               *      nothing, like any larger one: the LUTs are OpenCV's wherever OpenCV's own
+                               *      int conversion is defined, and huge or overflowing products clip nothing */
     int32_t tile_h, tile_w;   /* out: CLAHE tile size of the (reflect-extended) upscaled image */
     int32_t first_block;      /* out: index of this crop's first 32x32 output block in the batch */
     int32_t blocks_x;         /* out: output blocks per row */
@@ -397,7 +402,9 @@ int unetb200_enhance_plan(unetb200_enh_crop* table, int n, uint64_t* src_bytes, 
                           uint64_t* workspace_bytes);
 /* Enqueues the five kernels on `stream`.  table_host = the planned table (read for validation and grid
  * sizes), table_dev = the same n structs in device memory; src/out/workspace are device buffers of at
- * least the planned sizes.  Nothing is allocated; the workspace needs no initialisation. */
+ * least the planned sizes.  Nothing is allocated; the workspace needs no initialisation.  Before any CUDA
+ * call each crop of table_host is checked against what the plan gives (tiles, clip count, block grid,
+ * output and workspace offsets); a mismatch is EINVAL naming the crop and the field. */
 int unetb200_enhance_run(const unetb200_enh_crop* table_host, const void* table_dev, int n,
                          const uint8_t* src_dev, uint8_t* out_dev, void* workspace_dev, void* stream);
 

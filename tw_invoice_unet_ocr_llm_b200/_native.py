@@ -14,6 +14,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # UNETB200_LIB: load an alternative build of the same sources (A/B of compile-time switches); default in-tree
 LIB_PATH = os.environ.get("UNETB200_LIB") or os.path.join(_HERE, "libunetb200.so")
 
+# UNETB200_ABI_VERSION of include/unetb200.h: the structures below mirror that version's layouts
+ABI_VERSION = 2
 OK, EINVAL, ECUDA, EARCH, ENOMEM = 0, 1, 2, 3, 4
 STEM, CONV3X3, CONVT2X2, HEAD = 0, 1, 2, 3
 X_F32_NCHW, X_U8_NHWC, X_F16_NCHW, X_BF16_NCHW, X_F32_NHWC, X_F16_NHWC, X_BF16_NHWC = range(7)
@@ -44,7 +46,7 @@ class Layer(C.Structure):
 class EnhCrop(C.Structure):
     """``unetb200_enh_crop`` (include/unetb200.h): one crop of an enhancement batch."""
     _fields_ = [
-        ("h", C.c_int32), ("w", C.c_int32), ("flags", C.c_int32), ("clip", C.c_float),
+        ("h", C.c_int32), ("w", C.c_int32), ("flags", C.c_int32), ("clip", C.c_double),
         ("clip_count", C.c_int32), ("tile_h", C.c_int32), ("tile_w", C.c_int32),
         ("first_block", C.c_int32), ("blocks_x", C.c_int32), ("n_blocks", C.c_int32),
         ("src_stride", C.c_int32), ("src_pixel_bytes", C.c_int32),
@@ -145,6 +147,9 @@ def lib() -> C.CDLL:
                 fn = getattr(handle, name)
                 fn.restype = res
                 fn.argtypes = args
+            if handle.unetb200_abi_version() != ABI_VERSION:
+                raise RuntimeError(f"{LIB_PATH} has ABI version {handle.unetb200_abi_version()}, these bindings "
+                                   f"expect {ABI_VERSION}: rebuild it from this checkout")
             _lib = handle
     return _lib
 

@@ -1,12 +1,13 @@
 // C ABI of the OCR crop enhancement (include/unetb200.h, "OCR crop enhancement"); kernels in enhance.cuh.
 #include "enhance.cuh"
 
+#include <algorithm>
 #include <cmath>
 #include <cstdio>
 
 #include "errors.h"
 
-static_assert(sizeof(unetb200_enh_crop) == 72, "unetb200_enh_crop layout is part of the ABI");
+static_assert(sizeof(unetb200_enh_crop) == 80, "unetb200_enh_crop layout is part of the ABI");
 
 namespace {
 
@@ -33,10 +34,38 @@ constexpr int kMaxSide = 8192;          // 4x -> 32768: keeps every int product 
 
 bool crop_ok(const unetb200_enh_crop& c) {
     return c.h > 0 && c.w > 0 && c.h <= kMaxSide && c.w <= kMaxSide &&
-           (c.flags & ~(UNETB200_ENH_SHARPEN | UNETB200_ENH_BLUR | UNETB200_ENH_OTSU)) == 0 && c.clip > 0.f &&
+           (c.flags & ~(UNETB200_ENH_SHARPEN | UNETB200_ENH_BLUR | UNETB200_ENH_OTSU)) == 0 && c.clip > 0 &&
+           std::isfinite(c.clip) &&
            (c.src_stride == 0 || c.src_stride >= c.w) &&
            (c.src_pixel_bytes == 0 || c.src_pixel_bytes == 3 || c.src_pixel_bytes == 4) &&
            (c.src_stride != 0 || c.src_pixel_bytes != 4);          // packed crops are RGB
+}
+
+// what unetb200_enhance_plan derives from h, w and clip alone (enhance_run checks a table against it)
+struct EnhGeometry {
+    int tile_h, tile_w, clip_count, blocks_x, n_blocks;
+};
+
+EnhGeometry enh_geometry(const unetb200_enh_crop& c) {
+    const int H = 4 * c.h, W = 4 * c.w;
+    // CLAHE_Impl::apply: both dimensions are extended unless both divide the grid
+    int eh = H, ew = W;
+    if (H % ub::kEnhTiles != 0 || W % ub::kEnhTiles != 0) {
+        eh = H + (ub::kEnhTiles - H % ub::kEnhTiles);
+        ew = W + (ub::kEnhTiles - W % ub::kEnhTiles);
+    }
+    EnhGeometry g;
+    g.tile_h = eh / ub::kEnhTiles;
+    g.tile_w = ew / ub::kEnhTiles;
+    const int area = g.tile_h * g.tile_w;
+    // CLAHE_Impl::apply: (int)(clipLimit * tileSizeTotal / 256) in double.  No bin of a tile holds more than its
+    // area, so a limit at or above the area clips nothing, exactly like any larger one: clamping there keeps the
+    // conversion in range (huge or overflowing products) and the LUTs OpenCV's wherever its own int is defined.
+    const double limit = std::min(c.clip * area / 256, static_cast<double>(area));
+    g.clip_count = std::max(static_cast<int>(limit), 1);
+    g.blocks_x = (W + ub::kEnhBlock - 1) / ub::kEnhBlock;
+    g.n_blocks = g.blocks_x * ((H + ub::kEnhBlock - 1) / ub::kEnhBlock);
+    return g;
 }
 
 }  // namespace
@@ -54,23 +83,15 @@ int unetb200_enhance_plan(unetb200_enh_crop* table, int n, uint64_t* src_bytes, 
         if (!crop_ok(c)) {
             char buf[160];
             snprintf(buf, sizeof buf, "enhance_plan: crop %d invalid (h=%d w=%d flags=%d clip=%g)", i, c.h, c.w,
-                     c.flags, static_cast<double>(c.clip));
+                     c.flags, c.clip);
             return ub_fail(UNETB200_EINVAL, buf);
         }
-        const int H = 4 * c.h, W = 4 * c.w;
-        // CLAHE_Impl::apply: both dimensions are extended unless both divide the grid
-        int eh = H, ew = W;
-        if (H % ub::kEnhTiles != 0 || W % ub::kEnhTiles != 0) {
-            eh = H + (ub::kEnhTiles - H % ub::kEnhTiles);
-            ew = W + (ub::kEnhTiles - W % ub::kEnhTiles);
-        }
-        c.tile_h = eh / ub::kEnhTiles;
-        c.tile_w = ew / ub::kEnhTiles;
-        const int area = c.tile_h * c.tile_w;
-        int limit = static_cast<int>(static_cast<double>(c.clip) * area / 256);
-        c.clip_count = limit > 1 ? limit : 1;
-        c.blocks_x = (W + ub::kEnhBlock - 1) / ub::kEnhBlock;
-        c.n_blocks = c.blocks_x * ((H + ub::kEnhBlock - 1) / ub::kEnhBlock);
+        const EnhGeometry g = enh_geometry(c);
+        c.tile_h = g.tile_h;
+        c.tile_w = g.tile_w;
+        c.clip_count = g.clip_count;
+        c.blocks_x = g.blocks_x;
+        c.n_blocks = g.n_blocks;
         if (blocks + c.n_blocks > 0x7fffffff) return ub_fail(UNETB200_EINVAL, "enhance_plan: batch too large");
         c.first_block = static_cast<int32_t>(blocks);
         blocks += c.n_blocks;
@@ -98,21 +119,38 @@ int unetb200_enhance_run(const unetb200_enh_crop* table_host, const void* table_
     if ((reinterpret_cast<uintptr_t>(out_dev) | reinterpret_cast<uintptr_t>(workspace_dev) |
          reinterpret_cast<uintptr_t>(table_dev)) & 15)
         return ub_fail(UNETB200_EINVAL, "enhance_run: device buffers must be 16-byte aligned");
+    // the kernels index shared memory, LUTs and buffers by these fields: every one must be the plan's
     int64_t blocks = 0;
-    uint64_t out_bytes = 0;
+    uint64_t out_bytes = 0, ws_bytes = 0;
     bool any_otsu = false;
     for (int i = 0; i < n; ++i) {
         const unetb200_enh_crop& c = table_host[i];
-        if (!crop_ok(c) || c.src_stride < c.w || c.src_pixel_bytes == 0 || c.first_block != blocks || c.n_blocks <= 0 || c.tile_h <= 0 || c.tile_w <= 0 ||
-            c.blocks_x != (4 * c.w + ub::kEnhBlock - 1) / ub::kEnhBlock)
-            return ub_fail(UNETB200_EINVAL, "enhance_run: table was not produced by unetb200_enhance_plan");
-        if (c.out_off != out_bytes)
-            return ub_fail(UNETB200_EINVAL, "enhance_run: table was not produced by unetb200_enhance_plan");
+        const char* bad = nullptr;
+        if (!crop_ok(c)) {
+            bad = "h, w, flags, clip or source layout invalid";
+        } else {
+            const EnhGeometry g = enh_geometry(c);
+            if (c.src_stride < c.w || c.src_pixel_bytes == 0) bad = "src_stride / src_pixel_bytes not planned";
+            else if (c.tile_h != g.tile_h || c.tile_w != g.tile_w) bad = "tile_h / tile_w differ from the plan";
+            else if (c.clip_count != g.clip_count) bad = "clip_count differs from the plan";
+            else if (c.blocks_x != g.blocks_x || c.n_blocks != g.n_blocks)
+                bad = "blocks_x / n_blocks differ from the plan";
+            else if (c.first_block != blocks) bad = "first_block differs from the plan";
+            else if (c.out_off != out_bytes) bad = "out_off differs from the plan";
+            else if (c.ws_off != ws_bytes) bad = "ws_off differs from the plan";
+        }
+        if (bad) {
+            char buf[200];
+            snprintf(buf, sizeof buf, "enhance_run: crop %d: %s (table was not produced by unetb200_enhance_plan)",
+                     i, bad);
+            return ub_fail(UNETB200_EINVAL, buf);
+        }
         blocks += c.n_blocks;
         out_bytes += ub::enh_img_bytes(c.h, c.w);
+        ws_bytes += ub::enh_ws_bytes(c.h, c.w);
         any_otsu = any_otsu || (c.flags & UNETB200_ENH_OTSU);
     }
-    if (static_cast<int64_t>(n) * ub::kEnhTiles * ub::kEnhTiles > 0x7fffffff)
+    if (blocks > 0x7fffffff || static_cast<int64_t>(n) * ub::kEnhTiles * ub::kEnhTiles > 0x7fffffff)
         return ub_fail(UNETB200_EINVAL, "enhance_run: batch too large");
     static const ub::EnhTaps taps = cubic_taps_x4();
     cudaStream_t s = static_cast<cudaStream_t>(stream);

@@ -121,7 +121,7 @@ def enhance_batch(crops: Sequence, kinds: Sequence, device=None) -> List[Optiona
 def enhance_windows(frame: torch.Tensor, rects: Sequence[tuple], kinds: Sequence) -> List[np.ndarray]:
     """Enhance rectangles ``(x1, y1, x2, y2)`` (half-open) of a uint8 ``[H, W, 3]`` RGB (or ``[H, W, 4]``
     RGBX) frame that is already on the device -- the crops ``run_unet`` cuts from the frame it uploaded --
-    without packing or re-uploading them: only the 72-byte descriptors go up."""
+    without packing or re-uploading them: only the 80-byte descriptors go up."""
     if frame.dtype != torch.uint8 or frame.dim() != 3 or frame.shape[2] not in (3, 4) or not frame.is_cuda \
             or not frame.is_contiguous():
         raise RuntimeError("enhance_windows expects a contiguous CUDA uint8 [H,W,3] or [H,W,4] frame")
